@@ -2,6 +2,7 @@
 """bench.py -- the hot path's headline metric on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload config2|config3|config5]
+                    [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): stream-seconds of 48 kHz stereo analysed per second through the full
@@ -32,6 +33,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True            # the benchmark leaves the tree as it found it (no __pycache__)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "audio-analyzer-omega_b200"))
 
@@ -44,6 +46,7 @@ FLOP_TENSOR_FFT = 266240 + 122880         # the 8192 + 4096 FFTs of that estimat
 TENSOR_FLOP_PER_HOP = 3 * 2 * 960 * 512   # split-precision hop-block GEMM (three products): 960 columns x 512 samples per hop block
 FP32_PEAK_TFLOPS = 70.8                   # measured FFMA peak on this pool's B200 (profiles/r01_fp_pipes_microbench.txt:
                                           # 121.7 lanes/clk/SM x 148 SMs x 1.965 GHz x 2); nominal 75
+DUMP_ROWS = 16384                         # --dump-outputs: 16384 x (512 + 5) float32 = 34 MB at most
 
 
 def measured_peaks():
@@ -160,6 +163,19 @@ def bind_to_gpu_numa_node(local_rank, local_world):
     return info
 
 
+def dump_outputs(out_dir, comb, met):
+    """Write the same seeded sample of rows (row = channel * n_hops + hop) of the step's outputs ``comb``
+    [n_ch, n_hops, T] and ``met`` [n_ch, n_hops, 5] to out_dir/combined.npy and out_dir/meters.npy."""
+    import numpy as np
+    import torch
+    n_rows = comb.shape[0] * comb.shape[1]
+    rows = np.sort(np.random.default_rng(0).choice(n_rows, min(DUMP_ROWS, n_rows), replace=False))
+    idx = torch.from_numpy(rows).to(comb.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "combined.npy"), comb.reshape(n_rows, -1)[idx].cpu().numpy())
+    np.save(os.path.join(out_dir, "meters.npy"), met.reshape(n_rows, -1)[idx].cpu().numpy())
+
+
 def cpu_baseline(sample_seconds, streams=None, repeat=1):
     """Times oracle/ref_port.py (the reference's per-hop numpy/scipy path, a PORT pinned to the oracle) in a fresh
     interpreter on all host cores; returns (list of results, cores, streams)."""
@@ -222,7 +238,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the rank to its GPU's NUMA node")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0; config3: its last time "
+                         "tile) as DIR/combined.npy float32 [R, 512] and DIR/meters.npy float32 [R, 5]: the same "
+                         f"R <= {DUMP_ROWS} (channel, hop) rows of both, drawn with a fixed seed.  The input signal is "
+                         "seeded as well, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -311,33 +334,41 @@ def main():
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    launches0 = plan.launches
-    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    ktimes = {}
-    ev0.record()
-    for _ in range(args.steps):
-        step(N.FLAG_TIME_KERNELS)            # the library brackets each kernel with events on this stream
-    ev1.record()
-    barrier()
-    # kernel times of the last timed step's (last tile's) call (events of earlier calls are overwritten; same launches)
-    for name, ms in plan.kernel_times():
-        ktimes[name] = ms
-    launches = plan.launches - launches0
+    try:
+        launches0 = plan.launches
+        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        ktimes = {}
+        ev0.record()
+        for _ in range(args.steps):
+            step(N.FLAG_TIME_KERNELS)            # the library brackets each kernel with events on this stream
+        ev1.record()
+        barrier()
+        # kernel times of the last timed step's (last tile's) call (events of earlier calls are overwritten; same launches)
+        for name, ms in plan.kernel_times():
+            ktimes[name] = ms
+        launches = plan.launches - launches0
 
-    t_ms = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
-    if world > 1:
-        dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
-    clocks = sampler.stop() if rank == 0 else None
+        t_ms = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
+        if world > 1:
+            dist.all_reduce(t_ms, op=dist.ReduceOp.MAX)
+    finally:                                     # a failed step must not leave nvidia-smi running
+        clocks = sampler.stop() if rank == 0 else None
     total_ms = float(t_ms[0])
     ms_per_step = total_ms / args.steps
     stream_seconds_per_step = n_streams * seconds * world
     value = stream_seconds_per_step / (ms_per_step / 1e3)
 
+    # what the last timed step computed: the last tile's rows (config3's last tile may be shorter than the buffers)
+    last_n = tile_sizes[-1]
+    comb_out = comb if last_n == tile_hops else comb.view(-1)[:n_ch * last_n * T_BINS].view(n_ch, last_n, T_BINS)
+    met_out = met if last_n == tile_hops else met.view(-1)[:n_ch * last_n * N.N_METERS].view(n_ch, last_n, N.N_METERS)
+    if args.dump_outputs and rank == 0:          # before the e2e leg below reuses comb / met
+        dump_outputs(args.dump_outputs, comb_out, met_out)
+
     # the only collective of the whole path: gather the final per-stream rows (after the timed region):
     # the meters of the last hop + the last combined spectrum of every channel
-    last_n = tile_sizes[-1]
-    met_last = (met if last_n == tile_hops else met.view(-1)[:n_ch * last_n * N.N_METERS].view(n_ch, last_n, N.N_METERS))[:, -1, :]
-    comb_last = (comb if last_n == tile_hops else comb.view(-1)[:n_ch * last_n * T_BINS].view(n_ch, last_n, T_BINS))[:, -1, :]
+    met_last = met_out[:, -1, :]
+    comb_last = comb_out[:, -1, :]
     rows = torch.cat([met_last, comb_last], dim=1).reshape(n_streams, CHANNELS, N.N_METERS + T_BINS).contiguous()
     allrows = gather_rows(rows, n_streams * world) if world > 1 else rows
     checksum = float(allrows[..., :N.N_METERS].double().sum())

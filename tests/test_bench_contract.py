@@ -1,9 +1,12 @@
-"""bench.py contract checks that need no GPU: the reference arm's JSON line (the CPU port of the reference's path,
-a bounded sample per step) and the command-line surface the driver uses."""
+"""bench.py contract checks: the reference arm's JSON line (the CPU port of the reference's path, a bounded sample
+per step), the command-line surface the driver uses, and (on a GPU) the arrays --dump-outputs writes."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,6 +44,38 @@ def test_product_arm_refuses_to_run_without_a_gpu():
         pass
     out = _run("--steps", "1", "--no-cpu", "--no-e2e")
     assert out.returncode != 0 and "no CPU fallback" in (out.stderr + out.stdout)
+
+
+def test_steps_must_be_positive():
+    for impl in ("b200", "reference"):
+        out = _run("--impl", impl, "--steps", "0")
+        assert out.returncode != 0 and "--steps must be at least 1" in out.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_what_the_timed_step_computed(tmp_path):
+    """3 stereo streams x 2 s = 6 x 187 rows, fewer than the sample size: the dump is every row, in order, and equals
+    a separate analysis of the same seeded signal."""
+    import torch
+    sys.path.insert(0, os.path.join(ROOT, "audio-analyzer-omega_b200"))
+    from omega4_b200.batch.driver import analyze_resident, device_synth
+    from omega4_b200.plan import AnalysisPlan, BASELINE_CONFIGS
+    out = _run("--steps", "2", "--streams", "3", "--seconds", "2", "--no-cpu", "--no-e2e", "--dump-outputs", str(tmp_path))
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["combined.npy", "meters.npy"]
+    comb, met = np.load(tmp_path / "combined.npy"), np.load(tmp_path / "meters.npy")
+    n_ch, n_hops = 6, 2 * 48000 // 512
+    assert comb.dtype == met.dtype == np.float32 and comb.shape == (n_ch * n_hops, 512) and met.shape == (n_ch * n_hops, 5)
+    plan = AnalysisPlan(48000, BASELINE_CONFIGS, 512)
+    x = device_synth(3, 2, n_hops * 512)
+    want_c = torch.empty((n_ch, n_hops, 512), device="cuda")
+    want_m = torch.empty((n_ch, n_hops, 5), device="cuda")
+    analyze_resident(plan, x, combined=want_c, meters=want_m)
+    torch.cuda.synchronize()
+    assert np.array_equal(comb, want_c.reshape(-1, 512).cpu().numpy())
+    assert np.array_equal(met, want_m.reshape(-1, 5).cpu().numpy())
+    plan.close()
 
 
 def test_numa_binding_helper_is_harmless_without_topology():
