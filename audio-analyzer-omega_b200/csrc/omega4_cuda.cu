@@ -21,6 +21,7 @@
 #include "fft_core.cuh"
 #include "kweight_kernel.cuh"
 #include "kweight32_kernel.cuh"
+#include "loudness_kernel.cuh"
 #include "misc_kernels.cuh"
 #include "multires_kernel.cuh"
 #include "stats_kernel.cuh"
@@ -2150,6 +2151,162 @@ extern "C" int omega4_bars_run(omega4_bars* b, void* stream, int mem, const floa
         CK(cudaMemcpyAsync(band_values, d_out, rows * b->n_valid * sizeof(float), cudaMemcpyDeviceToHost, s));
         if (peak_values) CK(cudaMemcpyAsync(peak_values, d_peak, rows * b->n_valid * sizeof(float), cudaMemcpyDeviceToHost, s));
         if (state) CK(cudaMemcpyAsync(state, d_state, st_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return OMEGA4_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// ITU-R BS.1770-4 program loudness / EBU Tech 3342 loudness range (extension outside reference parity)
+// ------------------------------------------------------------------------------------------
+struct omega4_loudness {
+    int device = 0, fs = 0, C = 0, sub = 0;
+    double coef[10] = {};          // shelf b0 b1 b2 a1 a2, high-pass b0 b1 b2 a1 a2
+    double w[LOUD_MAX_CH] = {};
+    long long launches = 0;
+    DevBuf E, P, FS, Z;            // push scratch
+    DevBuf h_x, h_state, h_mom, h_st, h_peak, h_out;   // OMEGA4_MEM_HOST staging
+};
+
+extern "C" omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* d, int device) {
+    if (!d || !d->ch_weights || !d->shelf_b || !d->shelf_a || !d->hp_b || !d->hp_a) {
+        fail(OMEGA4_ERR_INVALID, "bad loudness descriptor"); return nullptr;
+    }
+    if (d->sample_rate <= 0 || d->sample_rate % 10 != 0 || d->sub != d->sample_rate / 10) {
+        fail(OMEGA4_ERR_INVALID, "sample rate must be a positive multiple of 10 and sub = sample_rate / 10"); return nullptr;
+    }
+    if (d->channels < 1 || d->channels > LOUD_MAX_CH) {
+        fail(OMEGA4_ERR_INVALID, "channels per stream must be 1 .. OMEGA4_LOUDNESS_MAX_CH"); return nullptr;
+    }
+    for (int c = 0; c < d->channels; ++c)
+        if (!(d->ch_weights[c] >= 0.0) || !isfinite(d->ch_weights[c])) {
+            fail(OMEGA4_ERR_INVALID, "channel weights must be finite and >= 0"); return nullptr;
+        }
+    const double* sec[4] = {d->shelf_b, d->shelf_a, d->hp_b, d->hp_a};
+    for (int i = 0; i < 4; ++i)
+        for (int j = 0; j < 3; ++j)
+            if (!isfinite(sec[i][j])) { fail(OMEGA4_ERR_INVALID, "K-weighting coefficients must be finite"); return nullptr; }
+    if (d->shelf_a[0] != 1.0 || d->hp_a[0] != 1.0) { fail(OMEGA4_ERR_INVALID, "biquads must be normalised (a[0] = 1)"); return nullptr; }
+    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
+    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    omega4_loudness* h = new omega4_loudness();
+    h->device = device; h->fs = d->sample_rate; h->C = d->channels; h->sub = d->sub;
+    const double q[10] = {d->shelf_b[0], d->shelf_b[1], d->shelf_b[2], d->shelf_a[1], d->shelf_a[2],
+                          d->hp_b[0], d->hp_b[1], d->hp_b[2], d->hp_a[1], d->hp_a[2]};
+    memcpy(h->coef, q, sizeof q);
+    for (int c = 0; c < d->channels; ++c) h->w[c] = d->ch_weights[c];
+    return h;
+}
+
+extern "C" void omega4_loudness_destroy(omega4_loudness* h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    for (DevBuf* b : {&h->E, &h->P, &h->FS, &h->Z, &h->h_x, &h->h_state, &h->h_mom, &h->h_st, &h->h_peak, &h->h_out})
+        b->release();
+    cudaGetLastError();
+    delete h;
+}
+
+extern "C" int omega4_loudness_state_doubles(const omega4_loudness* h) { return h ? loud_state_doubles(h->C) : 0; }
+
+extern "C" long long omega4_loudness_launches(const omega4_loudness* h) { return h ? h->launches : 0; }
+
+extern "C" int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, const float* samples, long long ch_stride,
+                                    int n_streams, long long n_samples, double* state, int fresh, long long out_stride,
+                                    float* momentary, float* short_term, float* sample_peak) {
+    if (!h || !samples || !state || n_streams < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
+        return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (n_streams == 0 || n_samples == 0) return OMEGA4_OK;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const int C = h->C, SD = loud_state_doubles(C);
+    const long long rows = (long long)n_streams * C;
+    const long long nsegb = n_samples / h->sub + 2;
+    if (nsegb > 2147483647LL / 32 || rows * nsegb > 2147483647LL * 4)
+        return fail(OMEGA4_ERR_INVALID, "push too large: split it into shorter tiles");
+    LoudArgs a;
+    memset(&a, 0, sizeof a);
+    a.x = samples; a.ch_stride = ch_stride; a.n = n_samples; a.n_streams = n_streams; a.C = C; a.sub = h->sub;
+    a.nsegb = (int)nsegb;
+    a.sb0 = h->coef[0]; a.sb1 = h->coef[1]; a.sb2 = h->coef[2]; a.sa1 = h->coef[3]; a.sa2 = h->coef[4];
+    a.hb0 = h->coef[5]; a.hb1 = h->coef[6]; a.hb2 = h->coef[7]; a.ha1 = h->coef[8]; a.ha2 = h->coef[9];
+    for (int c = 0; c < C; ++c) a.w[c] = h->w[c];
+    a.state = state; a.fresh = fresh ? 1 : 0;
+    a.mom = momentary; a.st = short_term; a.out_stride = out_stride; a.peak_db = sample_peak;
+    int rc;
+    if ((rc = h->E.ensure((size_t)rows * nsegb * sizeof(double)))) return rc;
+    if ((rc = h->P.ensure((size_t)rows * nsegb * sizeof(float)))) return rc;
+    if ((rc = h->FS.ensure((size_t)rows * 4 * sizeof(double)))) return rc;
+    if ((rc = h->Z.ensure((size_t)n_streams * nsegb * sizeof(double)))) return rc;
+    a.E = (double*)h->E.p; a.P = (float*)h->P.p; a.FS = (double*)h->FS.p; a.Z = (double*)h->Z.p;
+    long long ndone = 0;
+    const size_t st_bytes = (size_t)n_streams * SD * sizeof(double);
+    if (mem == OMEGA4_MEM_HOST) {
+        // host state is readable here: T is common to the streams of one state array
+        const long long T = fresh ? 0 : (long long)state[0];
+        ndone = (T + n_samples) / h->sub - T / h->sub;
+        if ((momentary || short_term) && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the step count");
+        if ((rc = h->h_x.ensure((size_t)rows * n_samples * sizeof(float)))) return rc;
+        if ((rc = h->h_state.ensure(st_bytes))) return rc;
+        CK(cudaMemcpy2DAsync(h->h_x.p, n_samples * sizeof(float), samples, ch_stride * sizeof(float),
+                             n_samples * sizeof(float), rows, cudaMemcpyHostToDevice, s));
+        if (!fresh) CK(cudaMemcpyAsync(h->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
+        a.x = (const float*)h->h_x.p; a.ch_stride = n_samples; a.state = (double*)h->h_state.p;
+        a.out_stride = ndone;
+        a.mom = a.st = nullptr; a.peak_db = nullptr;
+        if (momentary && ndone) { if ((rc = h->h_mom.ensure((size_t)n_streams * ndone * sizeof(float)))) return rc; a.mom = (float*)h->h_mom.p; }
+        if (short_term && ndone) { if ((rc = h->h_st.ensure((size_t)n_streams * ndone * sizeof(float)))) return rc; a.st = (float*)h->h_st.p; }
+        if (sample_peak) { if ((rc = h->h_peak.ensure((size_t)rows * sizeof(float)))) return rc; a.peak_db = (float*)h->h_peak.p; }
+    }
+    const long long warps = (rows * ((nsegb + LOUD_GROUP - 1) / LOUD_GROUP) + 31) / 32;
+    loudness_chain_kernel<<<(unsigned)((warps + LOUD_WARPS - 1) / LOUD_WARPS), LOUD_WARPS * 32, 0, s>>>(a);
+    CK(cudaGetLastError());
+    loudness_finalize_kernel<<<(unsigned)((n_streams + LOUD_WARPS - 1) / LOUD_WARPS), LOUD_WARPS * 32, 0, s>>>(a);
+    CK(cudaGetLastError());
+    h->launches += 2;
+    if (mem == OMEGA4_MEM_HOST) {
+        if (a.mom) CK(cudaMemcpy2DAsync(momentary, out_stride * sizeof(float), a.mom, ndone * sizeof(float),
+                                        ndone * sizeof(float), n_streams, cudaMemcpyDeviceToHost, s));
+        if (a.st) CK(cudaMemcpy2DAsync(short_term, out_stride * sizeof(float), a.st, ndone * sizeof(float),
+                                       ndone * sizeof(float), n_streams, cudaMemcpyDeviceToHost, s));
+        if (a.peak_db) CK(cudaMemcpyAsync(sample_peak, a.peak_db, (size_t)rows * sizeof(float), cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return OMEGA4_OK;
+}
+
+extern "C" int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem, const float* momentary,
+                                       const float* short_term, int n_streams, int n_steps, long long stride, float* out) {
+    if (!h || !momentary || !short_term || !out || n_streams < 0 || n_steps < 0 || stride < n_steps)
+        return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (n_streams == 0) return OMEGA4_OK;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const float* m = momentary; const float* st = short_term; float* o = out;
+    long long ld = stride;
+    if (mem == OMEGA4_MEM_HOST) {
+        const size_t bytes = (size_t)n_streams * (n_steps > 0 ? n_steps : 1) * sizeof(float);
+        int rc;
+        if ((rc = h->h_mom.ensure(bytes)) || (rc = h->h_st.ensure(bytes)) || (rc = h->h_out.ensure((size_t)n_streams * 4 * sizeof(float))))
+            return rc;
+        if (n_steps > 0) {
+            CK(cudaMemcpy2DAsync(h->h_mom.p, n_steps * sizeof(float), momentary, stride * sizeof(float),
+                                 n_steps * sizeof(float), n_streams, cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpy2DAsync(h->h_st.p, n_steps * sizeof(float), short_term, stride * sizeof(float),
+                                 n_steps * sizeof(float), n_streams, cudaMemcpyHostToDevice, s));
+        }
+        m = (const float*)h->h_mom.p; st = (const float*)h->h_st.p; o = (float*)h->h_out.p; ld = n_steps;
+    }
+    loudness_summary_kernel<<<(unsigned)n_streams, LOUD_SUM_THREADS, 0, s>>>(m, st, ld, n_steps, o);
+    CK(cudaGetLastError());
+    h->launches += 1;
+    if (mem == OMEGA4_MEM_HOST) {
+        CK(cudaMemcpyAsync(out, o, (size_t)n_streams * 4 * sizeof(float), cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
     }
     return OMEGA4_OK;

@@ -32,8 +32,9 @@ FLAG_TENSOR = 32
 FLAG_SERIAL_STATS = 64
 FLAG_FRESH_BARS = 128
 FLAG_EXACT_TRUE_PEAK = 256
-ABI_VERSION = 2
+ABI_VERSION = 3
 WATERFALL_STATE = 41
+LOUDNESS_MAX_CH = 32
 
 #: every symbol include/omega4_cuda.h declares (checked by tests/test_abi_symbols.py)
 EXPORTS = (
@@ -44,6 +45,8 @@ EXPORTS = (
     "omega4_analyze_s16", "omega4_plan_set_weighting", "omega4_bass_bars", "omega4_bars_create", "omega4_bars_destroy", "omega4_bars_count", "omega4_bars_run",
     "omega4_waterfall", "omega4_plan_set_gate_threshold",
     "omega4_analyze_io", "omega4_stream_hop", "omega4_meter_update",
+    "omega4_loudness_create", "omega4_loudness_destroy", "omega4_loudness_state_doubles",
+    "omega4_loudness_push", "omega4_loudness_summary", "omega4_loudness_launches",
 )
 
 
@@ -87,6 +90,16 @@ class BarsDesc(C.Structure):
         ("percentile", C.c_double),
         ("scale", C.c_float),
         ("normalize_max", C.c_int),
+    ]
+
+
+class LoudnessDesc(C.Structure):
+    """omega4_loudness_desc (include/omega4_cuda.h)."""
+    _fields_ = [
+        ("sample_rate", C.c_int), ("channels", C.c_int), ("ch_weights", C.POINTER(C.c_double)),
+        ("shelf_b", C.POINTER(C.c_double)), ("shelf_a", C.POINTER(C.c_double)),
+        ("hp_b", C.POINTER(C.c_double)), ("hp_a", C.POINTER(C.c_double)),
+        ("sub", C.c_int),
     ]
 
 
@@ -172,6 +185,18 @@ def lib() -> C.CDLL:
         l.omega4_bars_count.argtypes = [vp]
         l.omega4_bars_run.restype = ip
         l.omega4_bars_run.argtypes = [vp, vp, ip, vp, ip, ip, vp, ip, vp, vp]
+        l.omega4_loudness_create.restype = vp
+        l.omega4_loudness_create.argtypes = [C.POINTER(LoudnessDesc), ip]
+        l.omega4_loudness_destroy.restype = None
+        l.omega4_loudness_destroy.argtypes = [vp]
+        l.omega4_loudness_state_doubles.restype = ip
+        l.omega4_loudness_state_doubles.argtypes = [vp]
+        l.omega4_loudness_push.restype = ip
+        l.omega4_loudness_push.argtypes = [vp, vp, ip, vp, ll, ip, ll, vp, ip, ll, vp, vp, vp]
+        l.omega4_loudness_summary.restype = ip
+        l.omega4_loudness_summary.argtypes = [vp, vp, ip, vp, vp, ip, ip, ll, vp]
+        l.omega4_loudness_launches.restype = ll
+        l.omega4_loudness_launches.argtypes = [vp]
         if l.omega4_abi_version() != ABI_VERSION:
             raise Omega4CudaError(f"{LIB_NAME} ABI {l.omega4_abi_version()} != binding ABI {ABI_VERSION}")
         _lib = l

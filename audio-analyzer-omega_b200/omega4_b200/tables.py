@@ -207,3 +207,49 @@ def weighting_program(mode: str, sample_rate: int):
                              butter_lowhigh(2, min(f4 / nyq, 0.99) * nyq, sample_rate, "low")],
                 "blend": 0, "rms_gate": 1, "gain": 1.0}
     return {"sections": [], "blend": 0, "rms_gate": 0, "gain": 1.0}       # 'Z' and anything else (:228-229)
+
+
+# ------------------------------------------------------------------ ITU-R BS.1770-4 program loudness (extension)
+#: channel weights G_c per stream layout (BS.1770-4 Table 3; 5.1 in L R C LFE Ls Rs order, LFE excluded).
+#: There is no named 7.1 layout: its surround weights depend on speaker azimuth, so pass explicit weights.
+BS1770_LAYOUTS = {
+    "mono": (1.0,),
+    "stereo": (1.0, 1.0),
+    "5.1": (1.0, 1.0, 1.0, 0.0, 1.41, 1.41),
+}
+
+
+def bs1770_k_weighting(sample_rate: float) -> Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray]:
+    """(shelf_b, shelf_a, hp_b, hp_a), float64: the two K-weighting biquads of BS.1770-4 (high-shelf
+    pre-filter, then the RLB high-pass) for any sample rate, from the bilinear-transform closed form whose
+    parameters reproduce the standard's 48 kHz table to 1e-15."""
+    fs = float(sample_rate)
+    f0, G, Q = 1681.974450955533, 3.999843853973347, 0.7071752369554196
+    K = np.tan(np.pi * f0 / fs)
+    Vh = 10.0 ** (G / 20.0)
+    Vb = Vh ** 0.4996667741545416
+    a0 = 1.0 + K / Q + K * K
+    shelf_b = np.array([Vh + Vb * K / Q + K * K, 2.0 * (K * K - Vh), Vh - Vb * K / Q + K * K]) / a0
+    shelf_a = np.array([1.0, 2.0 * (K * K - 1.0) / a0, (1.0 - K / Q + K * K) / a0])
+    f0, Q = 38.13547087602444, 0.5003270373238773
+    K = np.tan(np.pi * f0 / fs)
+    d = 1.0 + K / Q + K * K
+    hp_b = np.array([1.0, -2.0, 1.0])
+    hp_a = np.array([1.0, 2.0 * (K * K - 1.0) / d, (1.0 - K / Q + K * K) / d])
+    return shelf_b, shelf_a, hp_b, hp_a
+
+
+def bs1770_channel_weights(layout_or_weights, n_channels: int | None = None) -> np.ndarray:
+    """float64 G_c from a layout name in ``BS1770_LAYOUTS`` or an explicit sequence of weights."""
+    if isinstance(layout_or_weights, str):
+        if layout_or_weights not in BS1770_LAYOUTS:
+            raise ValueError(f"unknown layout {layout_or_weights!r}: one of {sorted(BS1770_LAYOUTS)} "
+                             "or an explicit list of channel weights")
+        w = np.array(BS1770_LAYOUTS[layout_or_weights], dtype=np.float64)
+    else:
+        w = np.asarray(layout_or_weights, dtype=np.float64).reshape(-1)
+    if w.size < 1 or not np.all(np.isfinite(w)) or np.any(w < 0):
+        raise ValueError("channel weights must be one or more finite values >= 0")
+    if n_channels is not None and w.size != n_channels:
+        raise ValueError(f"{w.size} channel weights for {n_channels} channels")
+    return w

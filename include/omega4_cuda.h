@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define OMEGA4_ABI_VERSION 2
+#define OMEGA4_ABI_VERSION 3
 
 #define OMEGA4_OK 0
 #define OMEGA4_ERR_INVALID (-1)   /* bad argument */
@@ -298,6 +298,61 @@ int omega4_bars_count(const omega4_bars* bars);
  * NULL or fresh != 0 starts every channel without a previous frame. */
 int omega4_bars_run(omega4_bars* bars, void* stream, int mem, const float* spectrum, int n_ch, int n_hops,
                     float* state, int fresh, float* band_values, float* peak_values);
+
+/* ---- ITU-R BS.1770-4 program loudness and EBU Tech 3342 loudness range (extension) ---------- */
+/* Not part of the reference's behaviour: ProfessionalMetering (omega4_analyze's five meters) is not textbook
+ * BS.1770 and stays as it is.  This object measures, per stream of C planar channels, the K-weighted
+ * (high-shelf, then high-pass, run continuously from zero state) energy of every 100 ms sub-block of
+ * sub = sample_rate / 10 samples, z_j = sum_c G_c sum y_c^2, and from it
+ *   momentary  M_j = -0.691 + 10 log10(sum_{i=j-3..j} z_i / (4 sub))     NaN for j < 3
+ *   short-term S_j = -0.691 + 10 log10(sum_{i=j-29..j} z_i / (30 sub))   NaN for j < 29;  -inf for zero energy
+ * at the end of each sub-block j (counted from the stream start), the running sample peak per channel, and on
+ * request the integrated loudness (gated at -70 LUFS and 10 LU below) and the loudness range (short-term values
+ * gated at -70 and 20 LU below; v[floor(0.95 (n-1) + 0.5)] - v[floor(0.10 (n-1) + 0.5)] of the sorted survivors).
+ * DESIGN.md section 4.7.  One call at a time per object (it owns its scratch buffers). */
+#define OMEGA4_LOUDNESS_MAX_CH 32
+typedef struct omega4_loudness omega4_loudness;
+typedef struct omega4_loudness_desc {
+    int sample_rate;               /* a multiple of 10 */
+    int channels;                  /* C per stream, 1 .. OMEGA4_LOUDNESS_MAX_CH */
+    const double* ch_weights;      /* [channels] G_c >= 0 (1 1 for stereo; 1 1 1 0 1.41 1.41 for 5.1 L R C LFE Ls Rs) */
+    const double* shelf_b;         /* [3] K-weighting stage 1 (high-shelf), a[0] = 1 */
+    const double* shelf_a;
+    const double* hp_b;            /* [3] stage 2 (high-pass), a[0] = 1 */
+    const double* hp_a;
+    int sub;                       /* sample_rate / 10 */
+} omega4_loudness_desc;
+omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* desc, int device);
+void omega4_loudness_destroy(omega4_loudness* h);
+/* doubles of carried state per stream: 30 + 6 C (sample count, last 29 sub-block energies, per channel the
+ * filter state, the partial sub-block's energy and the sample peak) */
+int omega4_loudness_state_doubles(const omega4_loudness* h);
+/* Continue n_streams streams by n_samples samples each:
+ *   samples      [n_streams * C] planar rows (stream-major: row s * C + c), row r at samples + r * ch_stride
+ *   state        [n_streams][omega4_loudness_state_doubles] read (unless fresh) and written; every stream of one
+ *                state array has received the same number of samples T (each push advances all of them)
+ *   fresh        != 0: start every stream anew (T = 0), ignoring the contents of state
+ *   momentary, short_term  [n_streams][out_stride] float32 LUFS, or NULL: column i of row s receives step
+ *                floor(T / sub) + i of stream s.  A push of n samples after T emits
+ *                floor((T + n) / sub) - floor(T / sub) steps, so the caller knows the count without a sync.
+ *   sample_peak  [n_streams][C] float32 20 log10(max |x|) in dBFS over everything pushed since the start
+ *                (-inf for silence), or NULL
+ * Tile lengths are arbitrary (no multiple of sub or of 512 needed).  Values above -70 LUFS, the integrated loudness
+ * and the loudness range agree across tilings to ~1e-6 LU.  Far below the gate they may not: where digital silence
+ * follows a signal, a sub-block more than 100 ms into the silence reads either -inf (when the filter restarted from
+ * zero over a silent 100 ms warm-up) or a finite value below -120 LUFS (the filter's decaying ringing, when it
+ * continued from an earlier sub-block), and where the filter restarts depends on the push boundaries
+ * (DESIGN.md section 4.7). */
+int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, const float* samples, long long ch_stride,
+                         int n_streams, long long n_samples, double* state, int fresh, long long out_stride,
+                         float* momentary, float* short_term, float* sample_peak);
+/* momentary, short_term [n_streams][stride] series of n_steps steps each, counted from the stream start ->
+ * out [n_streams][4] float32: integrated loudness (-inf when no block passes the gates), loudness range (0 when no
+ * short-term value passes), max M, max S (NaN when n_steps leaves them undefined). */
+int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem, const float* momentary, const float* short_term,
+                            int n_streams, int n_steps, long long stride, float* out);
+/* number of kernels this library launched through `h` since creation (two per push, one per summary) */
+long long omega4_loudness_launches(const omega4_loudness* h);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* number of kernels this library launched through `plan` since creation */
