@@ -23,6 +23,7 @@
 #include "kweight32_kernel.cuh"
 #include "loudness_kernel.cuh"
 #include "misc_kernels.cuh"
+#include "octave_kernel.cuh"
 #include "multires_kernel.cuh"
 #include "stats_kernel.cuh"
 #include "truepeak_kernel.cuh"
@@ -2307,6 +2308,143 @@ extern "C" int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem
     h->launches += 1;
     if (mem == OMEGA4_MEM_HOST) {
         CK(cudaMemcpyAsync(out, o, (size_t)n_streams * 4 * sizeof(float), cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return OMEGA4_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// One-third-octave band levels per channel (extension outside reference parity)
+// ------------------------------------------------------------------------------------------
+struct omega4_octave {
+    int device = 0, fs = 0, nb = 0, sub = 0;
+    long long launches = 0;
+    DevBuf coef;                                   // [32][OCT_COEF] doubles
+    DevBuf h_x, h_state, h_levels, h_leq, h_lmax;  // OMEGA4_MEM_HOST staging
+};
+
+// zeros at z = 1 and z = -1 of a numerator g [1, -2, 1], g [1, 2, 1] or g [1, 0, -1]; false for anything else
+static bool oct_zero_pair(const double* b, int* plus, int* minus) {
+    if (!(b[0] != 0.0) || !isfinite(b[0])) return false;
+    if (b[1] == -2.0 * b[0] && b[2] == b[0]) { *plus += 2; return true; }
+    if (b[1] == 2.0 * b[0] && b[2] == b[0]) { *minus += 2; return true; }
+    if (b[1] == 0.0 && b[2] == -b[0]) { *plus += 1; *minus += 1; return true; }
+    return false;
+}
+
+extern "C" omega4_octave* omega4_octave_create(const omega4_octave_desc* d, int device) {
+    if (!d || !d->sos) { fail(OMEGA4_ERR_INVALID, "bad octave descriptor"); return nullptr; }
+    if (d->sample_rate < 8000 || d->sample_rate > 192000 || d->sample_rate % 10 != 0 || d->sub != d->sample_rate / 10) {
+        fail(OMEGA4_ERR_INVALID, "sample rate must be a multiple of 10 in [8000, 192000] and sub = sample_rate / 10");
+        return nullptr;
+    }
+    if (d->n_bands < 1 || d->n_bands > OCT_MAX_BANDS) {
+        fail(OMEGA4_ERR_INVALID, "n_bands must be 1 .. OMEGA4_OCTAVE_MAX_BANDS"); return nullptr;
+    }
+    double table[32 * OCT_COEF] = {};
+    for (int b = 0; b < d->n_bands; ++b) {
+        int plus = 0, minus = 0;
+        double g = 1.0;
+        for (int k = 0; k < 3; ++k) {
+            const double* s = d->sos + (b * 3 + k) * 6;
+            if (!oct_zero_pair(s, &plus, &minus)) {
+                fail(OMEGA4_ERR_INVALID, "octave section numerators must be g [1, -2, 1], g [1, 2, 1] or g [1, 0, -1]");
+                return nullptr;
+            }
+            const double a1 = s[4], a2 = s[5];
+            if (s[3] != 1.0 || !isfinite(a1) || !isfinite(a2) || !(fabs(a2) < 1.0) || !(fabs(a1) < 1.0 + a2)) {
+                fail(OMEGA4_ERR_INVALID, "octave sections must be normalised (a0 = 1) with poles inside the unit circle");
+                return nullptr;
+            }
+            g *= s[0];
+            table[b * OCT_COEF + 2 * k] = -a1;
+            table[b * OCT_COEF + 2 * k + 1] = -a2;
+        }
+        if (plus != 3 || minus != 3) {
+            fail(OMEGA4_ERR_INVALID, "each octave band needs three zeros at z = 1 and three at z = -1"); return nullptr;
+        }
+        table[b * OCT_COEF + 6] = 2.0 * g * g / d->sub;
+        table[b * OCT_COEF + 7] = 2.0 * g * g;
+    }
+    table[d->n_bands * OCT_COEF + 6] = 2.0 / d->sub;      // the overall column: no filter, unit gain
+    table[d->n_bands * OCT_COEF + 7] = 2.0;
+    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
+    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    omega4_octave* h = new omega4_octave();
+    h->device = device; h->fs = d->sample_rate; h->nb = d->n_bands; h->sub = d->sub;
+    const int rc = h->coef.ensure(sizeof table);          // sets the error message itself when it fails
+    if (rc != OMEGA4_OK || cudaMemcpy(h->coef.p, table, sizeof table, cudaMemcpyHostToDevice) != cudaSuccess) {
+        if (rc == OMEGA4_OK) fail(OMEGA4_ERR_CUDA, "copying the octave coefficients to the device failed");
+        omega4_octave_destroy(h);
+        return nullptr;
+    }
+    return h;
+}
+
+extern "C" void omega4_octave_destroy(omega4_octave* h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    for (DevBuf* b : {&h->coef, &h->h_x, &h->h_state, &h->h_levels, &h->h_leq, &h->h_lmax}) b->release();
+    cudaGetLastError();
+    delete h;
+}
+
+extern "C" int omega4_octave_state_doubles(const omega4_octave* h) { return h ? oct_state_doubles(h->nb) : 0; }
+
+extern "C" long long omega4_octave_launches(const omega4_octave* h) { return h ? h->launches : 0; }
+
+extern "C" int omega4_octave_push(omega4_octave* h, void* stream, int mem, const float* samples, long long ch_stride,
+                                  int n_rows, long long n_samples, double* state, int fresh, long long out_stride,
+                                  float* levels, float* leq, float* lmax) {
+    if (!h || !samples || !state || n_rows < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
+        return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (((uintptr_t)samples & 3) || ((uintptr_t)state & 7) || ((uintptr_t)levels & 3) || ((uintptr_t)leq & 3) ||
+        ((uintptr_t)lmax & 3))
+        return fail(OMEGA4_ERR_INVALID, "samples, levels, leq and lmax must be float-aligned and state double-aligned");
+    if (n_rows == 0 || n_samples == 0) return OMEGA4_OK;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    const int ncol = h->nb + 1, SD = oct_state_doubles(h->nb);
+    OctArgs a;
+    memset(&a, 0, sizeof a);
+    a.x = samples; a.ch_stride = ch_stride; a.n = n_samples; a.n_rows = n_rows; a.nb = h->nb; a.sub = h->sub;
+    a.coef = (const double*)h->coef.p;
+    a.state = state; a.fresh = fresh ? 1 : 0;
+    a.levels = levels; a.out_stride = out_stride; a.leq = leq; a.lmax = lmax;
+    long long ndone = 0;
+    const size_t st_bytes = (size_t)n_rows * SD * sizeof(double);
+    const size_t col_bytes = (size_t)n_rows * ncol * sizeof(float);
+    int rc;
+    if (mem == OMEGA4_MEM_HOST) {
+        // host state is readable here: T is common to the rows of one state array
+        const long long T = fresh ? 0 : (long long)state[0];
+        ndone = (T + n_samples) / h->sub - T / h->sub;
+        if (levels && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
+        if ((rc = h->h_x.ensure((size_t)n_rows * n_samples * sizeof(float)))) return rc;
+        if ((rc = h->h_state.ensure(st_bytes))) return rc;
+        CK(cudaMemcpy2DAsync(h->h_x.p, n_samples * sizeof(float), samples, ch_stride * sizeof(float),
+                             n_samples * sizeof(float), n_rows, cudaMemcpyHostToDevice, s));
+        if (!fresh) CK(cudaMemcpyAsync(h->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
+        a.x = (const float*)h->h_x.p; a.ch_stride = n_samples; a.state = (double*)h->h_state.p;
+        a.levels = nullptr; a.out_stride = ndone; a.leq = a.lmax = nullptr;
+        if (levels && ndone) {
+            if ((rc = h->h_levels.ensure((size_t)n_rows * ndone * ncol * sizeof(float)))) return rc;
+            a.levels = (float*)h->h_levels.p;
+        }
+        if (leq) { if ((rc = h->h_leq.ensure(col_bytes))) return rc; a.leq = (float*)h->h_leq.p; }
+        if (lmax) { if ((rc = h->h_lmax.ensure(col_bytes))) return rc; a.lmax = (float*)h->h_lmax.p; }
+    }
+    octave_kernel<<<(unsigned)((n_rows + OCT_WARPS - 1) / OCT_WARPS), OCT_WARPS * 32, 0, s>>>(a);
+    CK(cudaGetLastError());
+    h->launches += 1;
+    if (mem == OMEGA4_MEM_HOST) {
+        if (a.levels) CK(cudaMemcpy2DAsync(levels, out_stride * ncol * sizeof(float), a.levels, ndone * ncol * sizeof(float),
+                                           ndone * ncol * sizeof(float), n_rows, cudaMemcpyDeviceToHost, s));
+        if (a.leq) CK(cudaMemcpyAsync(leq, a.leq, col_bytes, cudaMemcpyDeviceToHost, s));
+        if (a.lmax) CK(cudaMemcpyAsync(lmax, a.lmax, col_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
     }
     return OMEGA4_OK;

@@ -32,9 +32,10 @@ FLAG_TENSOR = 32
 FLAG_SERIAL_STATS = 64
 FLAG_FRESH_BARS = 128
 FLAG_EXACT_TRUE_PEAK = 256
-ABI_VERSION = 3
+ABI_VERSION = 4
 WATERFALL_STATE = 41
 LOUDNESS_MAX_CH = 32
+OCTAVE_MAX_BANDS = 31
 
 #: every symbol include/omega4_cuda.h declares (checked by tests/test_abi_symbols.py)
 EXPORTS = (
@@ -47,6 +48,8 @@ EXPORTS = (
     "omega4_analyze_io", "omega4_stream_hop", "omega4_meter_update",
     "omega4_loudness_create", "omega4_loudness_destroy", "omega4_loudness_state_doubles",
     "omega4_loudness_push", "omega4_loudness_summary", "omega4_loudness_launches",
+    "omega4_octave_create", "omega4_octave_destroy", "omega4_octave_state_doubles", "omega4_octave_push",
+    "omega4_octave_launches",
 )
 
 
@@ -100,6 +103,13 @@ class LoudnessDesc(C.Structure):
         ("shelf_b", C.POINTER(C.c_double)), ("shelf_a", C.POINTER(C.c_double)),
         ("hp_b", C.POINTER(C.c_double)), ("hp_a", C.POINTER(C.c_double)),
         ("sub", C.c_int),
+    ]
+
+
+class OctaveDesc(C.Structure):
+    """omega4_octave_desc (include/omega4_cuda.h)."""
+    _fields_ = [
+        ("sample_rate", C.c_int), ("n_bands", C.c_int), ("sos", C.POINTER(C.c_double)), ("sub", C.c_int),
     ]
 
 
@@ -197,6 +207,16 @@ def lib() -> C.CDLL:
         l.omega4_loudness_summary.argtypes = [vp, vp, ip, vp, vp, ip, ip, ll, vp]
         l.omega4_loudness_launches.restype = ll
         l.omega4_loudness_launches.argtypes = [vp]
+        l.omega4_octave_create.restype = vp
+        l.omega4_octave_create.argtypes = [C.POINTER(OctaveDesc), ip]
+        l.omega4_octave_destroy.restype = None
+        l.omega4_octave_destroy.argtypes = [vp]
+        l.omega4_octave_state_doubles.restype = ip
+        l.omega4_octave_state_doubles.argtypes = [vp]
+        l.omega4_octave_push.restype = ip
+        l.omega4_octave_push.argtypes = [vp, vp, ip, vp, ll, ip, ll, vp, ip, ll, vp, vp, vp]
+        l.omega4_octave_launches.restype = ll
+        l.omega4_octave_launches.argtypes = [vp]
         if l.omega4_abi_version() != ABI_VERSION:
             raise Omega4CudaError(f"{LIB_NAME} ABI {l.omega4_abi_version()} != binding ABI {ABI_VERSION}")
         _lib = l

@@ -253,3 +253,65 @@ def bs1770_channel_weights(layout_or_weights, n_channels: int | None = None) -> 
     if n_channels is not None and w.size != n_channels:
         raise ValueError(f"{w.size} channel weights for {n_channels} channels")
     return w
+
+
+# ------------------------------------------------------------------ IEC 61260-1 one-third-octave bands (extension)
+#: nominal mid-band frequencies (Hz) of the base-10 bands x = -17 .. 13 (IEC 61260-1 Annex E)
+THIRD_OCTAVE_NOMINAL = (20, 25, 31.5, 40, 50, 63, 80, 100, 125, 160, 200, 250, 315, 400, 500, 630, 800,
+                        1000, 1250, 1600, 2000, 2500, 3150, 4000, 5000, 6300, 8000, 10000, 12500, 16000, 20000)
+THIRD_OCTAVE_X = tuple(range(-17, 14))
+THIRD_OCTAVE_ORDER = 3                     # Butterworth prototype order: a 6th-order band-pass, three biquads
+
+
+def check_octave_rate(sample_rate) -> int:
+    """The sample rate as an int; raises ValueError unless it is an integer multiple of 10 in [8000, 192000]
+    (100 ms blocks of fs / 10 samples)."""
+    try:
+        fs = int(sample_rate)
+    except (TypeError, ValueError):
+        raise ValueError(f"sample rate {sample_rate!r} must be an integer") from None
+    if fs != sample_rate or fs % 10 or not 8000 <= fs <= 192000:
+        raise ValueError(f"sample rate {sample_rate} must be an integer multiple of 10 in [8000, 192000]")
+    return fs
+
+
+def third_octave_bands(sample_rate) -> dict:
+    """The one-third-octave bands below Nyquist: base-10 system, exact mid-band f_m = 1000 * 10^(x / 10),
+    edges f_m * 10^(-/+ 1/20); a band is included iff its upper edge f2 < fs / 2 (31 bands at 48 and
+    96 kHz, 30 at 44.1 kHz, 23 at 8 kHz).  Returns float64 / int arrays ``x``, ``fm``, ``f1``, ``f2`` and
+    the nominal labels ``nominal``."""
+    fs = check_octave_rate(sample_rate)
+    x = np.array(THIRD_OCTAVE_X)
+    fm = 1000.0 * 10.0 ** (0.1 * x)
+    f1, f2 = fm * 10.0 ** -0.05, fm * 10.0 ** 0.05
+    keep = f2 < fs / 2.0
+    return {"x": x[keep], "fm": fm[keep], "f1": f1[keep], "f2": f2[keep],
+            "nominal": np.array(THIRD_OCTAVE_NOMINAL, dtype=np.float64)[keep]}
+
+
+def third_octave_sos(sample_rate) -> np.ndarray:
+    """[n_bands][3][6] float64 second-order sections (b0 b1 b2 1 a1 a2) of the digital Butterworth band-pass
+    of each band, the filter ``scipy.signal.butter(3, [f1, f2], btype="bandpass", fs=fs, output="sos")``
+    designs, in closed form: analog prototype poles, low-pass to band-pass on the pre-warped edges,
+    bilinear transform.  The arithmetic follows that design step for step (edges normalised to Nyquist,
+    pre-warped as 4 tan(pi Wn / 2), bilinear map z = (4 + s) / (4 - s)), so the coefficients agree with
+    scipy's to float64 rounding.  Each conjugate pole pair gets one zero pair (z = 1 and z = -1, numerator
+    g * [1, 0, -1]); the three sections share the gain equally.  The gain is 1/sqrt(2) at f1 and f2."""
+    fs = check_octave_rate(sample_rate)
+    b = third_octave_bands(fs)
+    N = THIRD_OCTAVE_ORDER
+    proto = -np.exp(1j * np.pi * np.arange(-N + 1, N, 2) / (2 * N))     # left half-plane unit-circle poles
+    sos = np.zeros((b["fm"].size, N, 6))
+    for i, (f1, f2) in enumerate(zip(b["f1"], b["f2"])):
+        w1, w2 = 4.0 * np.tan(np.pi * (2.0 * f1 / fs) / 2.0), 4.0 * np.tan(np.pi * (2.0 * f2 / fs) / 2.0)
+        bw, w0 = w2 - w1, np.sqrt(w1 * w2)
+        pl = proto * bw / 2.0
+        root = np.sqrt(pl ** 2 - w0 ** 2)
+        ps = np.concatenate([pl + root, pl - root])                        # 2N band-pass poles
+        pz = (4.0 + ps) / (4.0 - ps)
+        k = np.real(bw ** N * 4.0 ** N / np.prod(4.0 - ps))               # N zeros at s = 0, N at infinity
+        upper = np.sort_complex(pz[pz.imag > 0])
+        g = k ** (1.0 / N)
+        for j, p in enumerate(upper):
+            sos[i, j] = [g, 0.0, -g, 1.0, -(p + np.conj(p)).real, (p * np.conj(p)).real]
+    return sos

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define OMEGA4_ABI_VERSION 3
+#define OMEGA4_ABI_VERSION 4
 
 #define OMEGA4_OK 0
 #define OMEGA4_ERR_INVALID (-1)   /* bad argument */
@@ -353,6 +353,53 @@ int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem, const flo
                             int n_streams, int n_steps, long long stride, float* out);
 /* number of kernels this library launched through `h` since creation (two per push, one per summary) */
 long long omega4_loudness_launches(const omega4_loudness* h);
+
+/* ---- one-third-octave band levels per channel (IEC 61260-1 bands; extension) ----------------- */
+/* Not part of the reference's behaviour.  Per channel row: the base-10 one-third-octave bands x = -17 .. 13
+ * (f_m = 1000 * 10^(x/10) Hz, edges f_m * 10^(-/+0.05)) whose upper edge lies below fs / 2, each filtered by the
+ * 6th-order digital Butterworth band-pass that scipy.signal.butter(3, [f1, f2], "bandpass", fs=fs, output="sos")
+ * designs (-3.01 dB at the edges), run continuously over the whole stream from zero state in float64.  At the end
+ * of each 100 ms block j of sub = sample_rate / 10 samples (counted from the stream start) each band reads
+ *   L = 10 log10(2 / sub * sum_{n in j} y^2)   dBFS (a full-scale sine in the band reads 0 dBFS; -inf for zero energy)
+ * and column n_bands holds the same on the unfiltered input (the overall level).  Per row and column the object
+ * also keeps Leq = 10 log10(2 sum y^2 / T) over all T samples pushed (an incomplete last block included) and
+ * Lmax, the largest completed-block level; both -inf before any energy.  No channel summation, no weighting.
+ * The band frequencies follow IEC 61260-1; conformance to its filter class acceptance limits is not claimed.
+ * DESIGN.md section 4.8.  One call at a time per object (it owns its staging buffers). */
+#define OMEGA4_OCTAVE_MAX_BANDS 31
+typedef struct omega4_octave omega4_octave;
+typedef struct omega4_octave_desc {
+    int sample_rate;               /* a multiple of 10 in [8000, 192000] */
+    int n_bands;                   /* 1 .. OMEGA4_OCTAVE_MAX_BANDS */
+    const double* sos;             /* [n_bands][3][6] b0 b1 b2 a0 a1 a2 per section, a0 = 1, host memory, copied.  Each
+                                      band's numerators are g [1, -2, 1], g [1, 2, 1] or g [1, 0, -1] with three zeros at
+                                      z = 1 and three at z = -1 in all (scipy's pairing or tables.third_octave_sos); the
+                                      poles must lie inside the unit circle.  The kernel runs every section with
+                                      numerator [1, 0, -1] and applies the product of the b0 to the energy. */
+    int sub;                       /* sample_rate / 10 */
+} omega4_octave_desc;
+omega4_octave* omega4_octave_create(const omega4_octave_desc* desc, int device);
+void omega4_octave_destroy(omega4_octave* h);
+/* doubles of carried state per row: 1 + 9 (n_bands + 1) (the sample count T, then per column the 6 filter values,
+ * the partial block's energy, the energy of the completed blocks and the largest block energy) */
+int omega4_octave_state_doubles(const omega4_octave* h);
+/* Continue n_rows channel rows by n_samples samples each (one kernel launch):
+ *   samples   [n_rows] rows, row r at samples + r * ch_stride (ch_stride >= n_samples; float alignment suffices)
+ *   state     [n_rows][omega4_octave_state_doubles] doubles, read (unless fresh) and written; every row of one
+ *             state array has received the same number of samples T
+ *   fresh     != 0: start every row anew (T = 0), ignoring the contents of state
+ *   levels    [n_rows][out_stride][n_bands + 1] float32 dBFS, or NULL: column i of row r receives block
+ *             floor(T / sub) + i.  A push of n samples after T completes floor((T + n) / sub) - floor(T / sub)
+ *             blocks, so the caller knows the count without a sync; blocks at column >= out_stride are not written
+ *             (in host mode an out_stride below the count is an error).
+ *   leq, lmax [n_rows][n_bands + 1] float32 dBFS over everything pushed since the start, or NULL
+ * Tile lengths are arbitrary: the carried state is exact, so any cut of a stream into pushes gives bit-identical
+ * levels, Leq and Lmax. */
+int omega4_octave_push(omega4_octave* h, void* stream, int mem, const float* samples, long long ch_stride, int n_rows,
+                       long long n_samples, double* state, int fresh, long long out_stride, float* levels, float* leq,
+                       float* lmax);
+/* number of kernels this library launched through `h` since creation (one per push with samples) */
+long long omega4_octave_launches(const omega4_octave* h);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* number of kernels this library launched through `plan` since creation */
