@@ -2188,6 +2188,11 @@ extern "C" omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* d
         for (int j = 0; j < 3; ++j)
             if (!isfinite(sec[i][j])) { fail(OMEGA4_ERR_INVALID, "K-weighting coefficients must be finite"); return nullptr; }
     if (d->shelf_a[0] != 1.0 || d->hp_a[0] != 1.0) { fail(OMEGA4_ERR_INVALID, "biquads must be normalised (a[0] = 1)"); return nullptr; }
+    // the closed-form K-weighting is unstable at low rates (shelf poles outside the unit circle below ~4 kHz)
+    for (const double* a : {d->shelf_a, d->hp_a})
+        if (!(fabs(a[2]) < 1.0) || !(fabs(a[1]) < 1.0 + a[2])) {
+            fail(OMEGA4_ERR_INVALID, "K-weighting biquads must have their poles inside the unit circle"); return nullptr;
+        }
     if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
     if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
     omega4_loudness* h = new omega4_loudness();

@@ -84,10 +84,11 @@ __device__ __forceinline__ double st_percentile_f(const float* s, int n, double 
     return (t >= 0.5) ? (bv - d * (1.0 - t)) : (av + d * t);
 }
 
-// ONE WARP PER CHANNEL, no block barriers.  The per-frame values are rounded to float32 on entry
-// (the outputs are float32; 4e-6 LU) and every sum adds and subtracts exactly those rounded values
-// in double, so nothing drifts.  Shared memory per channel: the sorted gated copy and the ring of the last
-// 60 peaks only -- the window itself is never kept on chip: the value that expires from the 3600 / 180 / 24
+// ONE WARP PER CHANNEL, no block barriers.  The per-frame values are rounded to float32 for the sorted copy and
+// the sums (the outputs are float32; 4e-6 LU), and every sum adds and subtracts exactly those rounded values in
+// double, so nothing drifts.  Gate membership is decided on the unrounded double against the double gate, as the
+// reference does: a value in (-70, -70 + 3.8e-6) rounds to -70.0f but is a member.  Shared memory per channel:
+// the sorted gated copy and the ring of the last 60 peaks only -- the window itself is never kept on chip: the value that expires from the 3600 / 180 / 24
 // windows at hop k is the value pushed that many hops earlier, i.e. an element of the input series (or of
 // the carried state), fetched one 32-hop slice ahead with the new values.  14.7 KB per channel -> 15 channels
 // per SM: BASELINE's 2048 channels are resident in ONE wave (the kernel is a latency-bound sequential walk,
@@ -109,7 +110,6 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
     double* st = a.state + (size_t)ch * ST_STATE;
     const double* lufs = a.lufs + (size_t)ch * a.n_frames;
     const double* tps = a.tp + (size_t)ch * a.n_frames;
-    const float gate = (float)a.gate;
 
     int n_hist = 0, n_tp = 0;
     double cur[5] = {-100.0, -100.0, -100.0, 0.0, -100.0};
@@ -132,8 +132,8 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
     float tp_max = -CUDART_INF_F;
     if (CARRIED && (n_hist > 0 || n_tp > 0)) {                // carried state: rebuild the derived structures
         for (int i = lane; i < ST_SORT; i += 32) {
-            float v = (i < n_hist) ? (float)win0[i] : CUDART_INF_F;
-            srt[i] = (v > gate) ? v : CUDART_INF_F;           // non-gated entries sort to the end
+            const double v = (i < n_hist) ? win0[i] : 0.0;
+            srt[i] = (i < n_hist && v > a.gate) ? (float)v : CUDART_INF_F;   // non-gated entries sort to the end
         }
         __syncwarp();
         for (int k = 2; k <= ST_SORT; k <<= 1) {
@@ -150,7 +150,7 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
             }
         }
         double si = 0.0; int c = 0;
-        for (int i = lane; i < n_hist; i += 32) { float v = (float)win0[i]; if (v > gate) { ++c; si += (double)v; } }
+        for (int i = lane; i < n_hist; i += 32) { const double v = win0[i]; if (v > a.gate) { ++c; si += (double)(float)v; } }
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) { c += __shfl_xor_sync(0xffffffffu, c, o); si += __shfl_xor_sync(0xffffffffu, si, o); }
         ns = c; sum_i = si;
@@ -176,23 +176,27 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
     }
 
     // the value pushed D pushes before push p of this call: an element of the series, or of the carried window
-    auto pushed_before = [&](int p, int D) -> float {
+    auto pushed_before = [&](int p, int D) -> double {
         const int q = p - D;
-        if (q >= 0) return (float)lufs[kbeg + q];
+        if (q >= 0) return lufs[kbeg + q];
         const int c = n0 + q;
-        return (CARRIED && c >= 0) ? (float)win0[c] : 0.f;
+        return (CARRIED && c >= 0) ? win0[c] : 0.0;
     };
     float my_l = 0.f, my_t = 0.f, my_oi = 0.f, my_os = 0.f, my_om = 0.f;   // lane i holds hop kb + i of the current 32-hop slice
+    unsigned in_new = 0u;                                     // bit i: gate membership of the new value of hop kb + i
     for (int k = kbeg; k < a.n_frames; ++k) {
         const int kk = (k - kbeg) & 31;
         if (kk == 0) {
             const int idx = k + lane;
             const bool ok = idx < a.n_frames;
-            my_l = ok ? (float)lufs[idx] : 0.f;
+            const double l = ok ? lufs[idx] : 0.0;
+            const double oi = ok ? pushed_before(idx - kbeg, ST_I) : 0.0;  // leaves the 3600 window at this hop
+            my_l = (float)l;
             my_t = ok ? (float)tps[idx] : 0.f;
-            my_oi = ok ? pushed_before(idx - kbeg, ST_I) : 0.f;          // leaves the 3600 window at this hop
-            my_os = ok ? pushed_before(idx - kbeg, ST_S) : 0.f;          // leaves the 180 window
-            my_om = ok ? pushed_before(idx - kbeg, ST_M) : 0.f;          // leaves the 24 window
+            my_oi = (oi > a.gate) ? (float)oi : CUDART_NAN_F;              // NaN: not a gated member
+            my_os = ok ? (float)pushed_before(idx - kbeg, ST_S) : 0.f;     // leaves the 180 window
+            my_om = ok ? (float)pushed_before(idx - kbeg, ST_M) : 0.f;     // leaves the 24 window
+            in_new = __ballot_sync(0xffffffffu, ok && l > a.gate);
         }
         const float nv = __shfl_sync(0xffffffffu, my_l, kk);
         const float ntp = __shfl_sync(0xffffffffu, my_t, kk);
@@ -202,8 +206,8 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
         // ---- expiring value, positions in the sorted gated array
         const bool has_old = (n_hist == ST_I);
         const float ov = has_old ? ov_i : 0.f;
-        const bool rem = has_old && (ov > gate);
-        const bool ins = (nv > gate);
+        const bool rem = has_old && !isnan(ov);
+        const bool ins = (in_new >> kk) & 1u;
         const int prem = rem ? warp_lower_bound(srt, ns, ov, lane) : -1;
         const int pins = ins ? warp_lower_bound(srt, ns, nv, lane) : -1;   // position in the pre-removal array
         // ---- shift: remove old index prem, insert before old index pins
@@ -296,7 +300,7 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
             double v = 0.0;
             if (i < n_hist) {
                 const int c = i + shift;
-                v = (c < n0) ? (double)(float)win0[c] : (double)(float)lufs[kbeg + c - n0];
+                v = (c < n0) ? win0[c] : lufs[kbeg + c - n0];     // unrounded: a later call decides membership on it
             }
             __syncwarp();
             if (i < n_hist) st[8 + i] = v;
@@ -323,24 +327,25 @@ stats_kernel(const __grid_constant__ StatsArgs a) {
 // network, ~0.3 ms) to push a single value; here a 256-thread CTA per channel sorts the gated values of the new window
 // with block-wide steps (sort size = next power of two above the window length) and evaluates the statistics directly.
 // The per-frame values are rounded to float32 and summed in double exactly as above (those sums are exact, so the
-// order does not matter): the outputs are bit-identical to the walking kernel's.
+// order does not matter), and membership is decided on the unrounded values: the outputs are bit-identical to the
+// walking kernel's.  The window is kept in double for that (44.5 KB of static shared memory).
 // ---------------------------------------------------------------------------------------------
 constexpr int ST_P1_THREADS = 256;
 
 __global__ void __launch_bounds__(ST_P1_THREADS)
 stats_push1_kernel(const __grid_constant__ StatsArgs a) {
-    __shared__ float win[ST_I];                              // the new window, oldest first
+    __shared__ double win[ST_I];                             // the new window, oldest first, unrounded
     __shared__ float srt[ST_SORT];
     __shared__ float pk[ST_P];
     __shared__ double red_d[ST_P1_THREADS / 32];
     __shared__ int red_i[ST_P1_THREADS / 32];
     const int ch = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     double* st = a.state + (size_t)ch * ST_STATE;
-    const float gate = (float)a.gate;
     const int n0 = min(max((int)st[0], 0), ST_I), p0 = min(max((int)st[1], 0), ST_P);
-    const float nv = (float)a.lufs[ch], ntp = (float)a.tp[ch];
+    const double nv = a.lufs[ch];
+    const float ntp = (float)a.tp[ch];
     const int drop = (n0 == ST_I) ? 1 : 0, n = n0 - drop + 1;   // window after the push
-    for (int i = tid; i < n - 1; i += ST_P1_THREADS) win[i] = (float)st[8 + i + drop];
+    for (int i = tid; i < n - 1; i += ST_P1_THREADS) win[i] = st[8 + i + drop];
     const int pdrop = (p0 == ST_P) ? 1 : 0, np = p0 - pdrop + 1;
     for (int i = tid; i < np - 1; i += ST_P1_THREADS) pk[i] = (float)st[8 + ST_I + i + pdrop];
     if (tid == 0) { win[n - 1] = nv; pk[np - 1] = ntp; }
@@ -350,10 +355,11 @@ stats_push1_kernel(const __grid_constant__ StatsArgs a) {
     int c = 0;
     double si = 0.0;
     for (int i = tid; i < nsort; i += ST_P1_THREADS) {
-        const float v = (i < n) ? win[i] : CUDART_INF_F;
-        const bool g = v > gate && i < n;
-        srt[i] = g ? v : CUDART_INF_F;                        // non-gated entries sort to the end
-        if (g) { ++c; si += (double)v; }
+        const double v = (i < n) ? win[i] : 0.0;
+        const bool g = i < n && v > a.gate;
+        const float vf = (float)v;
+        srt[i] = g ? vf : CUDART_INF_F;                       // non-gated entries sort to the end
+        if (g) { ++c; si += (double)vf; }
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) { c += __shfl_xor_sync(0xffffffffu, c, o); si += __shfl_xor_sync(0xffffffffu, si, o); }
@@ -371,7 +377,7 @@ stats_push1_kernel(const __grid_constant__ StatsArgs a) {
             __syncthreads();
         }
     // new state: window and peak ring (every old value was copied to shared memory above)
-    for (int i = tid; i < n; i += ST_P1_THREADS) st[8 + i] = (double)win[i];
+    for (int i = tid; i < n; i += ST_P1_THREADS) st[8 + i] = win[i];
     for (int i = tid; i < np; i += ST_P1_THREADS) st[8 + ST_I + i] = (double)pk[i];
     if (tid == 0) {
         int ns = 0;
@@ -379,8 +385,8 @@ stats_push1_kernel(const __grid_constant__ StatsArgs a) {
         for (int w = 0; w < ST_P1_THREADS / 32; ++w) { ns += red_i[w]; sum_i += red_d[w]; }
         const int cm = n < ST_M ? n : ST_M, cs = n < ST_S ? n : ST_S;
         double sum_m = 0.0, sum_s = 0.0;
-        for (int i = n - cm; i < n; ++i) sum_m += (double)win[i];
-        for (int i = n - cs; i < n; ++i) sum_s += (double)win[i];
+        for (int i = n - cm; i < n; ++i) sum_m += (double)(float)win[i];
+        for (int i = n - cs; i < n; ++i) sum_s += (double)(float)win[i];
         float m = -CUDART_INF_F;
         for (int i = 0; i < np; ++i) m = fmaxf(m, pk[i]);
         double cur[5];

@@ -27,9 +27,15 @@ SUMMARY_KEYS = ("integrated", "lra", "max_momentary", "max_short_term")
 
 
 def _check_rate(sample_rate) -> int:
-    fs = int(sample_rate)
-    if fs != sample_rate or fs <= 0 or fs % 10:
-        raise ValueError(f"sample rate {sample_rate} must be a positive integer multiple of 10 (100 ms sub-blocks)")
+    """The sample rate as an int; raises ValueError unless it is an integer multiple of 10 (100 ms sub-blocks) in
+    [8000, 192000].  Below a few kHz the closed-form K-weighting shelf has poles outside the unit circle."""
+    try:
+        fs = int(sample_rate)
+    except (TypeError, ValueError):
+        raise ValueError(f"sample rate {sample_rate!r} must be an integer") from None
+    if fs != sample_rate or fs % 10 or not 8000 <= fs <= 192000:
+        raise ValueError(f"sample rate {sample_rate} must be an integer multiple of 10 in [8000, 192000] "
+                         "(100 ms sub-blocks)")
     return fs
 
 

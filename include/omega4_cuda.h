@@ -222,7 +222,8 @@ int omega4_meter_frames(omega4_plan* plan, void* stream, int mem,
                         const double* frames, int n_frames,
                         double* lufs_inst, double* tp_db, double* weighted);
 
-/* The deque statistics of calculate_lufs (professional_meters.py:248-279) over per-frame series. */
+/* The deque statistics of calculate_lufs (professional_meters.py:248-279) over per-frame series.
+ * Gate membership is decided on the float64 values; the sums and order statistics use them rounded to float32. */
 int omega4_meter_stats(omega4_plan* plan, void* stream, int mem,
                        const double* lufs_inst, const double* tp_db, int n_ch, int n_frames,
                        int first_frame, double* state, float* meters, int fresh);
@@ -313,7 +314,7 @@ int omega4_bars_run(omega4_bars* bars, void* stream, int mem, const float* spect
 #define OMEGA4_LOUDNESS_MAX_CH 32
 typedef struct omega4_loudness omega4_loudness;
 typedef struct omega4_loudness_desc {
-    int sample_rate;               /* a multiple of 10 */
+    int sample_rate;               /* a multiple of 10; both biquads must have their poles inside the unit circle */
     int channels;                  /* C per stream, 1 .. OMEGA4_LOUDNESS_MAX_CH */
     const double* ch_weights;      /* [channels] G_c >= 0 (1 1 for stereo; 1 1 1 0 1.41 1.41 for 5.1 L R C LFE Ls Rs) */
     const double* shelf_b;         /* [3] K-weighting stage 1 (high-shelf), a[0] = 1 */
