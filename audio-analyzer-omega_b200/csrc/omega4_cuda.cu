@@ -25,6 +25,7 @@
 #include "misc_kernels.cuh"
 #include "octave_kernel.cuh"
 #include "multires_kernel.cuh"
+#include "slm_kernel.cuh"
 #include "stats_kernel.cuh"
 #include "truepeak_kernel.cuh"
 #include "truepeak16_kernel.cuh"
@@ -2450,6 +2451,177 @@ extern "C" int omega4_octave_push(omega4_octave* h, void* stream, int mem, const
         if (a.leq) CK(cudaMemcpyAsync(leq, a.leq, col_bytes, cudaMemcpyDeviceToHost, s));
         if (a.lmax) CK(cudaMemcpyAsync(lmax, a.lmax, col_bytes, cudaMemcpyDeviceToHost, s));
         CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return OMEGA4_OK;
+}
+
+// ------------------------------------------------------------------------------------------
+// IEC 61672-1 sound level meter per channel (extension outside reference parity)
+// ------------------------------------------------------------------------------------------
+struct omega4_slm {
+    int device = 0, fs = 0, sub = 0;
+    long long launches = 0;
+    double aF = 0.0, aS = 0.0;
+    SlmCoef w[SLM_NW] = {};
+    DevBuf h_x, h_state, h_levels, h_totals, h_out;    // OMEGA4_MEM_HOST staging
+};
+
+// n_sec sections g [1, +-2, 1] with `plus` zeros at z = 1 and `minus` at z = -1 and stable poles -> c
+static bool slm_sections_ok(const double* sos, int n_sec, int plus, int minus, SlmCoef* c, const char** why) {
+    double g = 1.0;
+    int zp = 0, zm = 0;
+    for (int k = 0; k < n_sec; ++k) {
+        const double* s = sos + 6 * k;
+        if (!(s[0] != 0.0) || !isfinite(s[0]) || s[2] != s[0] || (s[1] != 2.0 * s[0] && s[1] != -2.0 * s[0])) {
+            *why = "weighting section numerators must be g [1, 2, 1] or g [1, -2, 1]"; return false;
+        }
+        const double a1 = s[4], a2 = s[5];
+        if (s[3] != 1.0 || !isfinite(a1) || !isfinite(a2) || !(fabs(a2) < 1.0) || !(fabs(a1) < 1.0 + a2)) {
+            *why = "weighting sections must be normalised (a0 = 1) with poles inside the unit circle"; return false;
+        }
+        const bool hp = s[1] == -2.0 * s[0];
+        (hp ? zp : zm) += 2;
+        c->m[k] = hp ? -2.0 : 2.0;
+        c->na1[k] = -a1;
+        c->na2[k] = -a2;
+        g *= s[0];
+    }
+    if (zp != plus || zm != minus) {
+        *why = "A needs four zeros at z = 1 and two at z = -1, C two and two"; return false;
+    }
+    c->g2 = g * g;
+    return true;
+}
+
+extern "C" omega4_slm* omega4_slm_create(const omega4_slm_desc* d, int device) {
+    if (!d || !d->sos_a || !d->sos_c) { fail(OMEGA4_ERR_INVALID, "bad sound level meter descriptor"); return nullptr; }
+    if (d->sample_rate < 8000 || d->sample_rate > 192000 || d->sample_rate % 10 != 0 || d->sub != d->sample_rate / 10) {
+        fail(OMEGA4_ERR_INVALID, "sample rate must be a multiple of 10 in [8000, 192000] and sub = sample_rate / 10");
+        return nullptr;
+    }
+    SlmCoef w[SLM_NW] = {};
+    const char* why = nullptr;
+    if (!slm_sections_ok(d->sos_a, 3, 4, 2, &w[0], &why) || !slm_sections_ok(d->sos_c, 2, 2, 2, &w[1], &why)) {
+        fail(OMEGA4_ERR_INVALID, why); return nullptr;
+    }
+    w[2].g2 = 1.0;                                          // Z: no filter
+    for (SlmCoef& c : w) c.g2_sub = c.g2 / d->sub;
+    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
+    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    omega4_slm* h = new omega4_slm();
+    h->device = device; h->fs = d->sample_rate; h->sub = d->sub;
+    h->aF = exp(-1.0 / (0.125 * d->sample_rate));
+    h->aS = exp(-1.0 / (1.0 * d->sample_rate));
+    memcpy(h->w, w, sizeof w);
+    return h;
+}
+
+extern "C" void omega4_slm_destroy(omega4_slm* h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    for (DevBuf* b : {&h->h_x, &h->h_state, &h->h_levels, &h->h_totals, &h->h_out}) b->release();
+    cudaGetLastError();
+    delete h;
+}
+
+extern "C" int omega4_slm_state_doubles(const omega4_slm* h) { return h ? SLM_STATE_DOUBLES : 0; }
+
+extern "C" long long omega4_slm_launches(const omega4_slm* h) { return h ? h->launches : 0; }
+
+extern "C" int omega4_slm_push(omega4_slm* h, void* stream, int mem, const float* samples, long long ch_stride,
+                               int n_rows, long long n_samples, double* state, int fresh, long long out_stride,
+                               float* levels, float* totals) {
+    if (!h || !samples || !state || n_rows < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
+        return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (((uintptr_t)samples & 3) || ((uintptr_t)state & 7) || ((uintptr_t)levels & 3) || ((uintptr_t)totals & 3))
+        return fail(OMEGA4_ERR_INVALID, "samples, levels and totals must be float-aligned and state double-aligned");
+    if (n_rows == 0 || n_samples == 0) return OMEGA4_OK;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    SlmArgs a;
+    memset(&a, 0, sizeof a);
+    a.x = samples; a.ch_stride = ch_stride; a.n = n_samples; a.n_rows = n_rows; a.sub = h->sub;
+    a.aF = h->aF; a.aS = h->aS;
+    memcpy(a.w, h->w, sizeof a.w);
+    a.state = state; a.fresh = fresh ? 1 : 0;
+    a.levels = levels; a.out_stride = out_stride; a.totals = totals;
+    long long ndone = 0;
+    const size_t st_bytes = (size_t)n_rows * SLM_STATE_DOUBLES * sizeof(double);
+    const size_t tot_bytes = (size_t)n_rows * SLM_NW * SLM_NTOT * sizeof(float);
+    const size_t blk_bytes = SLM_NCOL * sizeof(float);
+    int rc;
+    if (mem == OMEGA4_MEM_HOST) {
+        // host state is readable here: T is common to the rows of one state array
+        const long long T = fresh ? 0 : (long long)state[0];
+        ndone = (T + n_samples) / h->sub - T / h->sub;
+        if (levels && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
+        if ((rc = h->h_x.ensure((size_t)n_rows * n_samples * sizeof(float)))) return rc;
+        if ((rc = h->h_state.ensure(st_bytes))) return rc;
+        CK(cudaMemcpy2DAsync(h->h_x.p, n_samples * sizeof(float), samples, ch_stride * sizeof(float),
+                             n_samples * sizeof(float), n_rows, cudaMemcpyHostToDevice, s));
+        if (!fresh) CK(cudaMemcpyAsync(h->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
+        a.x = (const float*)h->h_x.p; a.ch_stride = n_samples; a.state = (double*)h->h_state.p;
+        a.levels = nullptr; a.out_stride = ndone; a.totals = nullptr;
+        if (levels && ndone) {
+            if ((rc = h->h_levels.ensure((size_t)n_rows * ndone * blk_bytes))) return rc;
+            a.levels = (float*)h->h_levels.p;
+        }
+        if (totals) { if ((rc = h->h_totals.ensure(tot_bytes))) return rc; a.totals = (float*)h->h_totals.p; }
+    }
+    slm_kernel<<<(unsigned)((n_rows + SLM_ROWS - 1) / SLM_ROWS), SLM_NW * 32, 0, s>>>(a);
+    CK(cudaGetLastError());
+    h->launches += 1;
+    if (mem == OMEGA4_MEM_HOST) {
+        if (a.levels) CK(cudaMemcpy2DAsync(levels, out_stride * blk_bytes, a.levels, ndone * blk_bytes, ndone * blk_bytes,
+                                           n_rows, cudaMemcpyDeviceToHost, s));
+        if (a.totals) CK(cudaMemcpyAsync(totals, a.totals, tot_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+    }
+    return OMEGA4_OK;
+}
+
+extern "C" int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, const float* levels, int n_rows,
+                                      int n_steps, long long stride, int column, int n_pct, const double* pct,
+                                      float* out) {
+    if (!h || !levels || !out || !pct || n_rows < 0 || n_steps < 0 || stride < n_steps)
+        return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (column < 0 || column >= SLM_NCOL) return fail(OMEGA4_ERR_INVALID, "column must be 0 .. 17");
+    if (n_pct < 1 || n_pct > SLM_MAX_PCT) return fail(OMEGA4_ERR_INVALID, "n_pct must be 1 .. OMEGA4_SLM_MAX_PCT");
+    if (((uintptr_t)levels & 3) || ((uintptr_t)out & 3))
+        return fail(OMEGA4_ERR_INVALID, "levels and out must be float-aligned");
+    SlmPctArgs a;
+    memset(&a, 0, sizeof a);
+    for (int p = 0; p < n_pct; ++p) {
+        const double N = pct[p];
+        if (!(N >= 0.0 && N <= 100.0)) return fail(OMEGA4_ERR_INVALID, "percentile N must be in [0, 100]");
+        // L_N = v[floor((1 - N / 100) (n - 1) + 0.5)] of the n values sorted ascending
+        a.rank[p] = n_steps ? (unsigned)floor((1.0 - N / 100.0) * (double)(n_steps - 1) + 0.5) : 0u;
+    }
+    if (n_rows == 0) return OMEGA4_OK;
+    CK(cudaSetDevice(h->device));
+    cudaStream_t s = (cudaStream_t)stream;
+    a.levels = levels; a.stride = stride; a.n_steps = n_steps; a.column = column; a.n_pct = n_pct; a.out = out;
+    const size_t out_bytes = (size_t)n_rows * n_pct * sizeof(float);
+    int rc;
+    if (mem == OMEGA4_MEM_HOST) {
+        const size_t row_bytes = (size_t)n_steps * SLM_NCOL * sizeof(float);
+        if ((rc = h->h_levels.ensure(n_steps ? (size_t)n_rows * row_bytes : sizeof(float)))) return rc;
+        if ((rc = h->h_out.ensure(out_bytes))) return rc;
+        if (n_steps) CK(cudaMemcpy2DAsync(h->h_levels.p, row_bytes, levels, (size_t)stride * SLM_NCOL * sizeof(float),
+                                          row_bytes, n_rows, cudaMemcpyHostToDevice, s));
+        a.levels = (const float*)h->h_levels.p; a.stride = n_steps; a.out = (float*)h->h_out.p;
+    }
+    slm_percentile_kernel<<<(unsigned)n_rows, SLM_PCT_THREADS, 0, s>>>(a);
+    CK(cudaGetLastError());
+    h->launches += 1;
+    if (mem == OMEGA4_MEM_HOST) {
+        CK(cudaMemcpyAsync(out, a.out, out_bytes, cudaMemcpyDeviceToHost, s));
         CK(cudaStreamSynchronize(s));
     }
     return OMEGA4_OK;

@@ -32,10 +32,11 @@ FLAG_TENSOR = 32
 FLAG_SERIAL_STATS = 64
 FLAG_FRESH_BARS = 128
 FLAG_EXACT_TRUE_PEAK = 256
-ABI_VERSION = 4
+ABI_VERSION = 5
 WATERFALL_STATE = 41
 LOUDNESS_MAX_CH = 32
 OCTAVE_MAX_BANDS = 31
+SLM_MAX_PCT = 64
 
 #: every symbol include/omega4_cuda.h declares (checked by tests/test_abi_symbols.py)
 EXPORTS = (
@@ -50,6 +51,8 @@ EXPORTS = (
     "omega4_loudness_push", "omega4_loudness_summary", "omega4_loudness_launches",
     "omega4_octave_create", "omega4_octave_destroy", "omega4_octave_state_doubles", "omega4_octave_push",
     "omega4_octave_launches",
+    "omega4_slm_create", "omega4_slm_destroy", "omega4_slm_state_doubles", "omega4_slm_push",
+    "omega4_slm_percentiles", "omega4_slm_launches",
 )
 
 
@@ -103,6 +106,13 @@ class LoudnessDesc(C.Structure):
         ("shelf_b", C.POINTER(C.c_double)), ("shelf_a", C.POINTER(C.c_double)),
         ("hp_b", C.POINTER(C.c_double)), ("hp_a", C.POINTER(C.c_double)),
         ("sub", C.c_int),
+    ]
+
+
+class SlmDesc(C.Structure):
+    """omega4_slm_desc (include/omega4_cuda.h)."""
+    _fields_ = [
+        ("sample_rate", C.c_int), ("sub", C.c_int), ("sos_a", C.POINTER(C.c_double)), ("sos_c", C.POINTER(C.c_double)),
     ]
 
 
@@ -217,6 +227,18 @@ def lib() -> C.CDLL:
         l.omega4_octave_push.argtypes = [vp, vp, ip, vp, ll, ip, ll, vp, ip, ll, vp, vp, vp]
         l.omega4_octave_launches.restype = ll
         l.omega4_octave_launches.argtypes = [vp]
+        l.omega4_slm_create.restype = vp
+        l.omega4_slm_create.argtypes = [C.POINTER(SlmDesc), ip]
+        l.omega4_slm_destroy.restype = None
+        l.omega4_slm_destroy.argtypes = [vp]
+        l.omega4_slm_state_doubles.restype = ip
+        l.omega4_slm_state_doubles.argtypes = [vp]
+        l.omega4_slm_push.restype = ip
+        l.omega4_slm_push.argtypes = [vp, vp, ip, vp, ll, ip, ll, vp, ip, ll, vp, vp]
+        l.omega4_slm_percentiles.restype = ip
+        l.omega4_slm_percentiles.argtypes = [vp, vp, ip, vp, ip, ip, ll, ip, ip, vp, vp]
+        l.omega4_slm_launches.restype = ll
+        l.omega4_slm_launches.argtypes = [vp]
         if l.omega4_abi_version() != ABI_VERSION:
             raise Omega4CudaError(f"{LIB_NAME} ABI {l.omega4_abi_version()} != binding ABI {ABI_VERSION}")
         _lib = l

@@ -315,3 +315,39 @@ def third_octave_sos(sample_rate) -> np.ndarray:
         for j, p in enumerate(upper):
             sos[i, j] = [g, 0.0, -g, 1.0, -(p + np.conj(p)).real, (p * np.conj(p)).real]
     return sos
+
+
+# ------------------------------------------------------------------ IEC 61672-1 frequency weightings (extension)
+#: pole frequencies f1 .. f4 (Hz) of the A and C weighting prototypes (IEC 61672-1 Annex E)
+IEC61672_POLE_HZ = (20.598997, 107.65265, 737.86223, 12194.217)
+
+
+def iec61672_weighting_sos(kind: str, sample_rate) -> np.ndarray:
+    """[n_sections][6] float64 second-order sections (b0 b1 b2 1 a1 a2) of the A (3 sections) or C (2 sections)
+    frequency weighting: the bilinear transform without pre-warping (``scipy.signal.bilinear_zpk``) of the
+    IEC 61672-1 Annex E prototype (A: four zeros at s = 0, poles at -2 pi {f1, f1, f2, f3, f4, f4}; C: two
+    zeros at s = 0, poles at -2 pi {f1, f1, f4, f4}), with the gain set so that |H| = 1 at 1 kHz.  In closed
+    form, numpy only: each real pole p maps to (2 fs + p) / (2 fs - p); zeros at s = 0 map to z = 1 and the
+    excess poles bring zeros at z = -1.  Sections in scipy's ``zpk2sos`` pairing: the f4 pair with
+    g [1, 2, 1], then (A only) the f2 / f3 pair and the f1 pair with g [1, -2, 1]; the sections share the
+    gain equally.  The design falls below the analog curve toward Nyquist (DESIGN.md section 4.9)."""
+    fs = check_octave_rate(sample_rate)
+    f1, f2, f3, f4 = IEC61672_POLE_HZ
+    if kind == "A":
+        plan = (((f4, f4), 2.0), ((f2, f3), -2.0), ((f1, f1), -2.0))
+    elif kind == "C":
+        plan = (((f4, f4), 2.0), ((f1, f1), -2.0))
+    else:
+        raise ValueError(f"weighting {kind!r} must be 'A' or 'C' (Z is no filter)")
+    fs2 = 2.0 * fs
+    z1 = np.exp(-2j * np.pi * 1000.0 / fs)                       # z^-1 at 1 kHz
+    sos = np.zeros((len(plan), 6))
+    h = 1.0 + 0j
+    for i, ((fa, fb), m) in enumerate(plan):
+        pa, pb = -2.0 * np.pi * fa, -2.0 * np.pi * fb
+        ra, rb = (fs2 + pa) / (fs2 - pa), (fs2 + pb) / (fs2 - pb)
+        sos[i] = [1.0, m, 1.0, 1.0, -(ra + rb), ra * rb]
+        h *= (1.0 + m * z1 + z1 * z1) / (1.0 + sos[i, 4] * z1 + sos[i, 5] * z1 * z1)
+    g = (1.0 / abs(h)) ** (1.0 / len(plan))
+    sos[:, :3] *= g
+    return sos

@@ -23,7 +23,7 @@
 extern "C" {
 #endif
 
-#define OMEGA4_ABI_VERSION 4
+#define OMEGA4_ABI_VERSION 5
 
 #define OMEGA4_OK 0
 #define OMEGA4_ERR_INVALID (-1)   /* bad argument */
@@ -401,6 +401,69 @@ int omega4_octave_push(omega4_octave* h, void* stream, int mem, const float* sam
                        float* lmax);
 /* number of kernels this library launched through `h` since creation (one per push with samples) */
 long long omega4_octave_launches(const omega4_octave* h);
+
+/* ---- IEC 61672-1 sound level meter per channel (extension) ------------------------------- */
+/* Not part of the reference's behaviour (its A / C / Z meters are frame-wise and unchanged).  Per channel row
+ * (rows are independent: no channel summation) and per frequency weighting W in the order A, C, Z:
+ *   A  the bilinear transform (no pre-warping) of the IEC 61672-1 Annex E prototype: four zeros at s = 0, poles at
+ *      -2 pi {f1, f1, f2, f3, f4, f4}, f1 = 20.598997, f2 = 107.65265, f3 = 737.86223, f4 = 12194.217 Hz, gain set so
+ *      |H| = 1 at 1 kHz: three biquads, one g [1, 2, 1] and two g [1, -2, 1];
+ *   C  the same with two zeros at s = 0 and poles -2 pi {f1, f1, f4, f4}: one g [1, 2, 1] and one g [1, -2, 1];
+ *   Z  no filter.
+ * Each filter runs continuously from zero state in float64.  With y the weighted signal and e_n = y_n^2, the time
+ * weightings v_n = a v_{n-1} + (1 - a) e_n, a = exp(-1 / (tau fs)), v_{-1} = 0, tau = 0.125 s (F) and 1 s (S), also
+ * run continuously in float64 (the meter starts from silence, so F and S read low for the first few tau).  Every
+ * level is 10 log10 of an energy in dB re a mean square of 1.0, -inf for zero (a full-scale sine reads Leq -3.01 dB
+ * and Lpeak 0 dB); add 20 log10(s / 20 uPa) for dB SPL when a sample of 1.0 is s pascal.
+ * Per 100 ms block j of sub = sample_rate / 10 samples (counted from the stream start), per weighting, in this order:
+ *   0 Leq = 10 log10(sum_{n in j} e_n / sub)      1 LFmax = max of v_F over the block   2 LSmax = max of v_S
+ *   3 LF = v_F at the block's last sample          4 LS = v_S there                      5 Lpeak = 20 log10 max |y_n|
+ * Totals per weighting over every sample pushed since the start (an incomplete last block included):
+ *   0 Leq = 10 log10(sum e / T)   1 LFmax   2 LSmax   3 Lpeak   (maxima over every pushed sample)
+ * DESIGN.md section 4.9.  One call at a time per object (it owns its staging buffers). */
+#define OMEGA4_SLM_WEIGHTINGS 3
+#define OMEGA4_SLM_QUANTITIES 6
+#define OMEGA4_SLM_TOTALS 4
+#define OMEGA4_SLM_MAX_PCT 64
+typedef struct omega4_slm omega4_slm;
+typedef struct omega4_slm_desc {
+    int sample_rate;               /* a multiple of 10 in [8000, 192000] */
+    int sub;                       /* sample_rate / 10 */
+    const double* sos_a;           /* [3][6] b0 b1 b2 a0 a1 a2, a0 = 1, host memory, copied: numerators g [1, +-2, 1] with
+                                      four zeros at z = 1 and two at z = -1 in all, poles inside the unit circle
+                                      (|a2| < 1, |a1| < 1 + a2); tables.iec61672_weighting_sos("A", fs) */
+    const double* sos_c;           /* [2][6] the same for C: two zeros at z = 1 and two at z = -1 */
+} omega4_slm_desc;
+omega4_slm* omega4_slm_create(const omega4_slm_desc* desc, int device);
+void omega4_slm_destroy(omega4_slm* h);
+/* doubles of carried state per row: 41 (the sample count T; per weighting the filter values (6, 4, 0), v_F, v_S,
+ * the partial block's energy and its maxima of v_F, v_S and e, the completed blocks' energy and their maxima) */
+int omega4_slm_state_doubles(const omega4_slm* h);
+/* Continue n_rows channel rows by n_samples samples each (one kernel launch):
+ *   samples   [n_rows] rows, row r at samples + r * ch_stride (ch_stride >= n_samples; float alignment suffices)
+ *   state     [n_rows][omega4_slm_state_doubles] doubles, read (unless fresh) and written; every row of one state
+ *             array has received the same number of samples T
+ *   fresh     != 0: start every row anew (T = 0), ignoring the contents of state
+ *   levels    [n_rows][out_stride][3][6] float32 dB (weighting A, C, Z; quantity as above), or NULL: column i of row
+ *             r receives block floor(T / sub) + i.  A push of n samples after T completes floor((T + n) / sub) -
+ *             floor(T / sub) blocks; blocks at column >= out_stride are not written (in host mode an out_stride
+ *             below the count is an error).
+ *   totals    [n_rows][3][4] float32 dB over everything pushed since the start, or NULL
+ * Tile lengths are arbitrary: the carried state is exact, so any cut of a stream into pushes gives bit-identical
+ * levels, totals and state. */
+int omega4_slm_push(omega4_slm* h, void* stream, int mem, const float* samples, long long ch_stride, int n_rows,
+                    long long n_samples, double* state, int fresh, long long out_stride, float* levels, float* totals);
+/* Percentile levels of one series column (one kernel launch): for each row r the first n_steps values
+ * levels[r][j][column / 6][column % 6] (levels [n_rows][stride][3][6], stride >= n_steps, column 0 .. 17) sorted
+ * ascending as v, and for each of the n_pct (1 .. OMEGA4_SLM_MAX_PCT) values N = pct[p] in [0, 100] (host memory)
+ *   out[r][p] = L_N = v[floor((1 - N / 100) (n_steps - 1) + 0.5)]
+ * the level exceeded N % of the time: L_0 is the maximum, L_100 the minimum, -inf counts as the lowest value, NaN
+ * for n_steps = 0.  Exact order statistics of the stored float32 values. */
+int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, const float* levels, int n_rows, int n_steps,
+                           long long stride, int column, int n_pct, const double* pct, float* out);
+/* number of kernels this library launched through `h` since creation (one per push with samples, one per
+ * percentile query with rows) */
+long long omega4_slm_launches(const omega4_slm* h);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* number of kernels this library launched through `plan` since creation */
