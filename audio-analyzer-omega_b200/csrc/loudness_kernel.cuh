@@ -184,8 +184,8 @@ __global__ void __launch_bounds__(LOUD_WARPS * 32) loudness_finalize_kernel(Loud
         }
         const float M = j >= 3 ? loud_lufs(sm * inv4) : CUDART_NAN_F;
         const float S = j >= LOUD_HIST ? loud_lufs(ss * inv30) : CUDART_NAN_F;
-        if (a.mom) a.mom[s * a.out_stride + jl] = M;
-        if (a.st) a.st[s * a.out_stride + jl] = S;
+        if (a.mom && jl < a.out_stride) a.mom[s * a.out_stride + jl] = M;
+        if (a.st && jl < a.out_stride) a.st[s * a.out_stride + jl] = S;
     }
     // carried state: every read of the old state above happens before any write below
     double h = 0.0;

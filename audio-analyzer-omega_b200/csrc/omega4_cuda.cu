@@ -9,6 +9,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <set>
@@ -2159,6 +2160,111 @@ extern "C" int omega4_bars_run(omega4_bars* b, void* stream, int mem, const floa
 }
 
 // ------------------------------------------------------------------------------------------
+// block meters (loudness, one-third-octave, sound level meter): the host side their calls share
+// ------------------------------------------------------------------------------------------
+// create: a meter object needs a device, made current here
+static bool meter_device(int device) {
+    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return false; }
+    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return false; }
+    return true;
+}
+
+static int check_mem(int mem) {
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    return OMEGA4_OK;
+}
+
+// the push arguments every block meter takes (include/omega4_cuda.h); `outs` are its float outputs, null or not
+static int check_push(const void* h, int mem, const float* samples, long long ch_stride, int n_rows,
+                      long long n_samples, const double* state, long long out_stride,
+                      std::initializer_list<const float*> outs) {
+    if (!h || !samples || !state || n_rows < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
+        return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
+    bool aligned = !((uintptr_t)samples & 3) && !((uintptr_t)state & 7);
+    for (const float* p : outs) aligned = aligned && !((uintptr_t)p & 3);
+    if (!aligned) return fail(OMEGA4_ERR_INVALID, "samples and outputs must be float-aligned and state double-aligned");
+    return OMEGA4_OK;
+}
+
+// OMEGA4_MEM_HOST staging of one call: its host inputs go to device buffers the meter keeps (they only grow), the
+// kernels run on those, and finish() copies the outputs and the state back and synchronises once.  Sizes and
+// pitches are in floats.
+struct HostStage {
+    struct Back { float* dst; long long dpitch; const float* src; long long width, rows; };
+    DevBuf buf[5];                 // slot k holds the k-th array a call stages; a push with three outputs uses all
+    Back back[3];
+    int nbuf = 0, nback = 0;
+    cudaStream_t s = nullptr;
+    double* state = nullptr;       // host state to copy back, from state_dev
+    const double* state_dev = nullptr;
+    size_t state_bytes = 0;
+
+    void begin(cudaStream_t stream) { s = stream; nbuf = nback = 0; state = nullptr; }
+
+    // the block count of a push of n samples: floor((T + n) / sub) - floor(T / sub), with T = state[0] common to
+    // the rows of one state array and readable on the host
+    static long long blocks(const double* st, int fresh, long long n, int sub) {
+        const long long T = fresh ? 0 : (long long)st[0];
+        return (T + n) / sub - T / sub;
+    }
+
+    // rows x width floats at src (row pitch spitch) -> a dense device copy
+    int in(const float* src, long long spitch, long long width, long long rows, const float** dev) {
+        DevBuf& b = buf[nbuf++];
+        const size_t bytes = (size_t)(width * rows) * sizeof(float);
+        if (int rc = b.ensure(bytes ? bytes : sizeof(float))) return rc;
+        if (bytes) CK(cudaMemcpy2DAsync(b.p, width * sizeof(float), src, spitch * sizeof(float), width * sizeof(float),
+                                        rows, cudaMemcpyHostToDevice, s));
+        *dev = (const float*)b.p;
+        return OMEGA4_OK;
+    }
+
+    // a device buffer of rows x width floats that finish() copies to dst (row pitch dpitch); nullptr when dst is
+    // null or there is nothing to write
+    int out(float* dst, long long dpitch, long long width, long long rows, float** dev) {
+        DevBuf& b = buf[nbuf++];
+        *dev = nullptr;
+        if (!dst || width * rows == 0) return OMEGA4_OK;
+        if (int rc = b.ensure((size_t)(width * rows) * sizeof(float))) return rc;
+        *dev = (float*)b.p;
+        back[nback++] = {dst, dpitch, *dev, width, rows};
+        return OMEGA4_OK;
+    }
+
+    // a push's inputs: the samples [rows][n] (row pitch *ch_stride) densely, and the carried state (copied in
+    // unless fresh, back at finish()); the pointers and the stride are replaced by the device ones
+    int push(const float** x, long long* ch_stride, long long rows, long long n, double** st, size_t st_bytes,
+             int fresh) {
+        if (int rc = in(*x, *ch_stride, n, rows, x)) return rc;
+        *ch_stride = n;
+        DevBuf& b = buf[nbuf++];
+        if (int rc = b.ensure(st_bytes)) return rc;
+        if (!fresh) CK(cudaMemcpyAsync(b.p, *st, st_bytes, cudaMemcpyHostToDevice, s));
+        state = *st; state_dev = (const double*)b.p; state_bytes = st_bytes;
+        *st = (double*)b.p;
+        return OMEGA4_OK;
+    }
+
+    int finish() {
+        for (int i = 0; i < nback; ++i) {
+            const Back& c = back[i];
+            if (c.dpitch == c.width)
+                CK(cudaMemcpyAsync(c.dst, c.src, (size_t)(c.width * c.rows) * sizeof(float), cudaMemcpyDeviceToHost, s));
+            else
+                CK(cudaMemcpy2DAsync(c.dst, c.dpitch * sizeof(float), c.src, c.width * sizeof(float),
+                                     c.width * sizeof(float), c.rows, cudaMemcpyDeviceToHost, s));
+        }
+        if (state) CK(cudaMemcpyAsync(state, state_dev, state_bytes, cudaMemcpyDeviceToHost, s));
+        CK(cudaStreamSynchronize(s));
+        return OMEGA4_OK;
+    }
+
+    void release() { for (DevBuf& b : buf) b.release(); }
+};
+
+// ------------------------------------------------------------------------------------------
 // ITU-R BS.1770-4 program loudness / EBU Tech 3342 loudness range (extension outside reference parity)
 // ------------------------------------------------------------------------------------------
 struct omega4_loudness {
@@ -2167,7 +2273,7 @@ struct omega4_loudness {
     double w[LOUD_MAX_CH] = {};
     long long launches = 0;
     DevBuf E, P, FS, Z;            // push scratch
-    DevBuf h_x, h_state, h_mom, h_st, h_peak, h_out;   // OMEGA4_MEM_HOST staging
+    HostStage stage;
 };
 
 extern "C" omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* d, int device) {
@@ -2194,8 +2300,7 @@ extern "C" omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* d
         if (!(fabs(a[2]) < 1.0) || !(fabs(a[1]) < 1.0 + a[2])) {
             fail(OMEGA4_ERR_INVALID, "K-weighting biquads must have their poles inside the unit circle"); return nullptr;
         }
-    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
-    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    if (!meter_device(device)) return nullptr;
     omega4_loudness* h = new omega4_loudness();
     h->device = device; h->fs = d->sample_rate; h->C = d->channels; h->sub = d->sub;
     const double q[10] = {d->shelf_b[0], d->shelf_b[1], d->shelf_b[2], d->shelf_a[1], d->shelf_a[2],
@@ -2208,8 +2313,8 @@ extern "C" omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* d
 extern "C" void omega4_loudness_destroy(omega4_loudness* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    for (DevBuf* b : {&h->E, &h->P, &h->FS, &h->Z, &h->h_x, &h->h_state, &h->h_mom, &h->h_st, &h->h_peak, &h->h_out})
-        b->release();
+    for (DevBuf* b : {&h->E, &h->P, &h->FS, &h->Z}) b->release();
+    h->stage.release();
     cudaGetLastError();
     delete h;
 }
@@ -2221,10 +2326,9 @@ extern "C" long long omega4_loudness_launches(const omega4_loudness* h) { return
 extern "C" int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, const float* samples, long long ch_stride,
                                     int n_streams, long long n_samples, double* state, int fresh, long long out_stride,
                                     float* momentary, float* short_term, float* sample_peak) {
-    if (!h || !samples || !state || n_streams < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
-        return fail(OMEGA4_ERR_INVALID, "bad arguments");
-    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (int rc = check_push(h, mem, samples, ch_stride, n_streams, n_samples, state, out_stride,
+                            {momentary, short_term, sample_peak}))
+        return rc;
     if (n_streams == 0 || n_samples == 0) return OMEGA4_OK;
     CK(cudaSetDevice(h->device));
     cudaStream_t s = (cudaStream_t)stream;
@@ -2248,24 +2352,18 @@ extern "C" int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, c
     if ((rc = h->FS.ensure((size_t)rows * 4 * sizeof(double)))) return rc;
     if ((rc = h->Z.ensure((size_t)n_streams * nsegb * sizeof(double)))) return rc;
     a.E = (double*)h->E.p; a.P = (float*)h->P.p; a.FS = (double*)h->FS.p; a.Z = (double*)h->Z.p;
-    long long ndone = 0;
-    const size_t st_bytes = (size_t)n_streams * SD * sizeof(double);
+    HostStage& hs = h->stage;
     if (mem == OMEGA4_MEM_HOST) {
-        // host state is readable here: T is common to the streams of one state array
-        const long long T = fresh ? 0 : (long long)state[0];
-        ndone = (T + n_samples) / h->sub - T / h->sub;
-        if ((momentary || short_term) && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the step count");
-        if ((rc = h->h_x.ensure((size_t)rows * n_samples * sizeof(float)))) return rc;
-        if ((rc = h->h_state.ensure(st_bytes))) return rc;
-        CK(cudaMemcpy2DAsync(h->h_x.p, n_samples * sizeof(float), samples, ch_stride * sizeof(float),
-                             n_samples * sizeof(float), rows, cudaMemcpyHostToDevice, s));
-        if (!fresh) CK(cudaMemcpyAsync(h->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
-        a.x = (const float*)h->h_x.p; a.ch_stride = n_samples; a.state = (double*)h->h_state.p;
+        const long long ndone = HostStage::blocks(state, fresh, n_samples, h->sub);
+        if ((momentary || short_term) && out_stride < ndone)
+            return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
+        hs.begin(s);
+        if ((rc = hs.push(&a.x, &a.ch_stride, rows, n_samples, &a.state, (size_t)n_streams * SD * sizeof(double), fresh)) ||
+            (rc = hs.out(momentary, out_stride, ndone, n_streams, &a.mom)) ||
+            (rc = hs.out(short_term, out_stride, ndone, n_streams, &a.st)) ||
+            (rc = hs.out(sample_peak, rows, rows, 1, &a.peak_db)))
+            return rc;
         a.out_stride = ndone;
-        a.mom = a.st = nullptr; a.peak_db = nullptr;
-        if (momentary && ndone) { if ((rc = h->h_mom.ensure((size_t)n_streams * ndone * sizeof(float)))) return rc; a.mom = (float*)h->h_mom.p; }
-        if (short_term && ndone) { if ((rc = h->h_st.ensure((size_t)n_streams * ndone * sizeof(float)))) return rc; a.st = (float*)h->h_st.p; }
-        if (sample_peak) { if ((rc = h->h_peak.ensure((size_t)rows * sizeof(float)))) return rc; a.peak_db = (float*)h->h_peak.p; }
     }
     const long long warps = (rows * ((nsegb + LOUD_GROUP - 1) / LOUD_GROUP) + 31) / 32;
     loudness_chain_kernel<<<(unsigned)((warps + LOUD_WARPS - 1) / LOUD_WARPS), LOUD_WARPS * 32, 0, s>>>(a);
@@ -2273,50 +2371,32 @@ extern "C" int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, c
     loudness_finalize_kernel<<<(unsigned)((n_streams + LOUD_WARPS - 1) / LOUD_WARPS), LOUD_WARPS * 32, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 2;
-    if (mem == OMEGA4_MEM_HOST) {
-        if (a.mom) CK(cudaMemcpy2DAsync(momentary, out_stride * sizeof(float), a.mom, ndone * sizeof(float),
-                                        ndone * sizeof(float), n_streams, cudaMemcpyDeviceToHost, s));
-        if (a.st) CK(cudaMemcpy2DAsync(short_term, out_stride * sizeof(float), a.st, ndone * sizeof(float),
-                                       ndone * sizeof(float), n_streams, cudaMemcpyDeviceToHost, s));
-        if (a.peak_db) CK(cudaMemcpyAsync(sample_peak, a.peak_db, (size_t)rows * sizeof(float), cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
 }
 
 extern "C" int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem, const float* momentary,
                                        const float* short_term, int n_streams, int n_steps, long long stride, float* out) {
     if (!h || !momentary || !short_term || !out || n_streams < 0 || n_steps < 0 || stride < n_steps)
         return fail(OMEGA4_ERR_INVALID, "bad arguments");
-    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (int rc = check_mem(mem)) return rc;
     if (n_streams == 0) return OMEGA4_OK;
     CK(cudaSetDevice(h->device));
     cudaStream_t s = (cudaStream_t)stream;
     const float* m = momentary; const float* st = short_term; float* o = out;
     long long ld = stride;
+    HostStage& hs = h->stage;
     if (mem == OMEGA4_MEM_HOST) {
-        const size_t bytes = (size_t)n_streams * (n_steps > 0 ? n_steps : 1) * sizeof(float);
+        hs.begin(s);
         int rc;
-        if ((rc = h->h_mom.ensure(bytes)) || (rc = h->h_st.ensure(bytes)) || (rc = h->h_out.ensure((size_t)n_streams * 4 * sizeof(float))))
+        if ((rc = hs.in(momentary, stride, n_steps, n_streams, &m)) ||
+            (rc = hs.in(short_term, stride, n_steps, n_streams, &st)) || (rc = hs.out(out, 4, 4, n_streams, &o)))
             return rc;
-        if (n_steps > 0) {
-            CK(cudaMemcpy2DAsync(h->h_mom.p, n_steps * sizeof(float), momentary, stride * sizeof(float),
-                                 n_steps * sizeof(float), n_streams, cudaMemcpyHostToDevice, s));
-            CK(cudaMemcpy2DAsync(h->h_st.p, n_steps * sizeof(float), short_term, stride * sizeof(float),
-                                 n_steps * sizeof(float), n_streams, cudaMemcpyHostToDevice, s));
-        }
-        m = (const float*)h->h_mom.p; st = (const float*)h->h_st.p; o = (float*)h->h_out.p; ld = n_steps;
+        ld = n_steps;
     }
     loudness_summary_kernel<<<(unsigned)n_streams, LOUD_SUM_THREADS, 0, s>>>(m, st, ld, n_steps, o);
     CK(cudaGetLastError());
     h->launches += 1;
-    if (mem == OMEGA4_MEM_HOST) {
-        CK(cudaMemcpyAsync(out, o, (size_t)n_streams * 4 * sizeof(float), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -2326,7 +2406,7 @@ struct omega4_octave {
     int device = 0, fs = 0, nb = 0, sub = 0;
     long long launches = 0;
     DevBuf coef;                                   // [32][OCT_COEF] doubles
-    DevBuf h_x, h_state, h_levels, h_leq, h_lmax;  // OMEGA4_MEM_HOST staging
+    HostStage stage;
 };
 
 // zeros at z = 1 and z = -1 of a numerator g [1, -2, 1], g [1, 2, 1] or g [1, 0, -1]; false for anything else
@@ -2374,8 +2454,7 @@ extern "C" omega4_octave* omega4_octave_create(const omega4_octave_desc* d, int 
     }
     table[d->n_bands * OCT_COEF + 6] = 2.0 / d->sub;      // the overall column: no filter, unit gain
     table[d->n_bands * OCT_COEF + 7] = 2.0;
-    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
-    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    if (!meter_device(device)) return nullptr;
     omega4_octave* h = new omega4_octave();
     h->device = device; h->fs = d->sample_rate; h->nb = d->n_bands; h->sub = d->sub;
     const int rc = h->coef.ensure(sizeof table);          // sets the error message itself when it fails
@@ -2390,7 +2469,8 @@ extern "C" omega4_octave* omega4_octave_create(const omega4_octave_desc* d, int 
 extern "C" void omega4_octave_destroy(omega4_octave* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    for (DevBuf* b : {&h->coef, &h->h_x, &h->h_state, &h->h_levels, &h->h_leq, &h->h_lmax}) b->release();
+    h->coef.release();
+    h->stage.release();
     cudaGetLastError();
     delete h;
 }
@@ -2402,13 +2482,8 @@ extern "C" long long omega4_octave_launches(const omega4_octave* h) { return h ?
 extern "C" int omega4_octave_push(omega4_octave* h, void* stream, int mem, const float* samples, long long ch_stride,
                                   int n_rows, long long n_samples, double* state, int fresh, long long out_stride,
                                   float* levels, float* leq, float* lmax) {
-    if (!h || !samples || !state || n_rows < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
-        return fail(OMEGA4_ERR_INVALID, "bad arguments");
-    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
-    if (((uintptr_t)samples & 3) || ((uintptr_t)state & 7) || ((uintptr_t)levels & 3) || ((uintptr_t)leq & 3) ||
-        ((uintptr_t)lmax & 3))
-        return fail(OMEGA4_ERR_INVALID, "samples, levels, leq and lmax must be float-aligned and state double-aligned");
+    if (int rc = check_push(h, mem, samples, ch_stride, n_rows, n_samples, state, out_stride, {levels, leq, lmax}))
+        return rc;
     if (n_rows == 0 || n_samples == 0) return OMEGA4_OK;
     CK(cudaSetDevice(h->device));
     cudaStream_t s = (cudaStream_t)stream;
@@ -2419,41 +2494,23 @@ extern "C" int omega4_octave_push(omega4_octave* h, void* stream, int mem, const
     a.coef = (const double*)h->coef.p;
     a.state = state; a.fresh = fresh ? 1 : 0;
     a.levels = levels; a.out_stride = out_stride; a.leq = leq; a.lmax = lmax;
-    long long ndone = 0;
-    const size_t st_bytes = (size_t)n_rows * SD * sizeof(double);
-    const size_t col_bytes = (size_t)n_rows * ncol * sizeof(float);
-    int rc;
+    HostStage& hs = h->stage;
     if (mem == OMEGA4_MEM_HOST) {
-        // host state is readable here: T is common to the rows of one state array
-        const long long T = fresh ? 0 : (long long)state[0];
-        ndone = (T + n_samples) / h->sub - T / h->sub;
+        const long long ndone = HostStage::blocks(state, fresh, n_samples, h->sub);
         if (levels && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
-        if ((rc = h->h_x.ensure((size_t)n_rows * n_samples * sizeof(float)))) return rc;
-        if ((rc = h->h_state.ensure(st_bytes))) return rc;
-        CK(cudaMemcpy2DAsync(h->h_x.p, n_samples * sizeof(float), samples, ch_stride * sizeof(float),
-                             n_samples * sizeof(float), n_rows, cudaMemcpyHostToDevice, s));
-        if (!fresh) CK(cudaMemcpyAsync(h->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
-        a.x = (const float*)h->h_x.p; a.ch_stride = n_samples; a.state = (double*)h->h_state.p;
-        a.levels = nullptr; a.out_stride = ndone; a.leq = a.lmax = nullptr;
-        if (levels && ndone) {
-            if ((rc = h->h_levels.ensure((size_t)n_rows * ndone * ncol * sizeof(float)))) return rc;
-            a.levels = (float*)h->h_levels.p;
-        }
-        if (leq) { if ((rc = h->h_leq.ensure(col_bytes))) return rc; a.leq = (float*)h->h_leq.p; }
-        if (lmax) { if ((rc = h->h_lmax.ensure(col_bytes))) return rc; a.lmax = (float*)h->h_lmax.p; }
+        hs.begin(s);
+        const long long cols = (long long)n_rows * ncol;
+        int rc;
+        if ((rc = hs.push(&a.x, &a.ch_stride, n_rows, n_samples, &a.state, (size_t)n_rows * SD * sizeof(double), fresh)) ||
+            (rc = hs.out(levels, out_stride * ncol, ndone * ncol, n_rows, &a.levels)) ||
+            (rc = hs.out(leq, cols, cols, 1, &a.leq)) || (rc = hs.out(lmax, cols, cols, 1, &a.lmax)))
+            return rc;
+        a.out_stride = ndone;
     }
     octave_kernel<<<(unsigned)((n_rows + OCT_WARPS - 1) / OCT_WARPS), OCT_WARPS * 32, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 1;
-    if (mem == OMEGA4_MEM_HOST) {
-        if (a.levels) CK(cudaMemcpy2DAsync(levels, out_stride * ncol * sizeof(float), a.levels, ndone * ncol * sizeof(float),
-                                           ndone * ncol * sizeof(float), n_rows, cudaMemcpyDeviceToHost, s));
-        if (a.leq) CK(cudaMemcpyAsync(leq, a.leq, col_bytes, cudaMemcpyDeviceToHost, s));
-        if (a.lmax) CK(cudaMemcpyAsync(lmax, a.lmax, col_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -2464,7 +2521,7 @@ struct omega4_slm {
     long long launches = 0;
     double aF = 0.0, aS = 0.0;
     SlmCoef w[SLM_NW] = {};
-    DevBuf h_x, h_state, h_levels, h_totals, h_out;    // OMEGA4_MEM_HOST staging
+    HostStage stage;
 };
 
 // n_sec sections g [1, +-2, 1] with `plus` zeros at z = 1 and `minus` at z = -1 and stable poles -> c
@@ -2507,8 +2564,7 @@ extern "C" omega4_slm* omega4_slm_create(const omega4_slm_desc* d, int device) {
     }
     w[2].g2 = 1.0;                                          // Z: no filter
     for (SlmCoef& c : w) c.g2_sub = c.g2 / d->sub;
-    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
-    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    if (!meter_device(device)) return nullptr;
     omega4_slm* h = new omega4_slm();
     h->device = device; h->fs = d->sample_rate; h->sub = d->sub;
     h->aF = exp(-1.0 / (0.125 * d->sample_rate));
@@ -2520,7 +2576,7 @@ extern "C" omega4_slm* omega4_slm_create(const omega4_slm_desc* d, int device) {
 extern "C" void omega4_slm_destroy(omega4_slm* h) {
     if (!h) return;
     cudaSetDevice(h->device);
-    for (DevBuf* b : {&h->h_x, &h->h_state, &h->h_levels, &h->h_totals, &h->h_out}) b->release();
+    h->stage.release();
     cudaGetLastError();
     delete h;
 }
@@ -2532,12 +2588,8 @@ extern "C" long long omega4_slm_launches(const omega4_slm* h) { return h ? h->la
 extern "C" int omega4_slm_push(omega4_slm* h, void* stream, int mem, const float* samples, long long ch_stride,
                                int n_rows, long long n_samples, double* state, int fresh, long long out_stride,
                                float* levels, float* totals) {
-    if (!h || !samples || !state || n_rows < 0 || n_samples < 0 || ch_stride < n_samples || out_stride < 0)
-        return fail(OMEGA4_ERR_INVALID, "bad arguments");
-    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
-    if (((uintptr_t)samples & 3) || ((uintptr_t)state & 7) || ((uintptr_t)levels & 3) || ((uintptr_t)totals & 3))
-        return fail(OMEGA4_ERR_INVALID, "samples, levels and totals must be float-aligned and state double-aligned");
+    if (int rc = check_push(h, mem, samples, ch_stride, n_rows, n_samples, state, out_stride, {levels, totals}))
+        return rc;
     if (n_rows == 0 || n_samples == 0) return OMEGA4_OK;
     CK(cudaSetDevice(h->device));
     cudaStream_t s = (cudaStream_t)stream;
@@ -2548,40 +2600,24 @@ extern "C" int omega4_slm_push(omega4_slm* h, void* stream, int mem, const float
     memcpy(a.w, h->w, sizeof a.w);
     a.state = state; a.fresh = fresh ? 1 : 0;
     a.levels = levels; a.out_stride = out_stride; a.totals = totals;
-    long long ndone = 0;
-    const size_t st_bytes = (size_t)n_rows * SLM_STATE_DOUBLES * sizeof(double);
-    const size_t tot_bytes = (size_t)n_rows * SLM_NW * SLM_NTOT * sizeof(float);
-    const size_t blk_bytes = SLM_NCOL * sizeof(float);
-    int rc;
+    HostStage& hs = h->stage;
     if (mem == OMEGA4_MEM_HOST) {
-        // host state is readable here: T is common to the rows of one state array
-        const long long T = fresh ? 0 : (long long)state[0];
-        ndone = (T + n_samples) / h->sub - T / h->sub;
+        const long long ndone = HostStage::blocks(state, fresh, n_samples, h->sub);
         if (levels && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
-        if ((rc = h->h_x.ensure((size_t)n_rows * n_samples * sizeof(float)))) return rc;
-        if ((rc = h->h_state.ensure(st_bytes))) return rc;
-        CK(cudaMemcpy2DAsync(h->h_x.p, n_samples * sizeof(float), samples, ch_stride * sizeof(float),
-                             n_samples * sizeof(float), n_rows, cudaMemcpyHostToDevice, s));
-        if (!fresh) CK(cudaMemcpyAsync(h->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
-        a.x = (const float*)h->h_x.p; a.ch_stride = n_samples; a.state = (double*)h->h_state.p;
-        a.levels = nullptr; a.out_stride = ndone; a.totals = nullptr;
-        if (levels && ndone) {
-            if ((rc = h->h_levels.ensure((size_t)n_rows * ndone * blk_bytes))) return rc;
-            a.levels = (float*)h->h_levels.p;
-        }
-        if (totals) { if ((rc = h->h_totals.ensure(tot_bytes))) return rc; a.totals = (float*)h->h_totals.p; }
+        hs.begin(s);
+        const long long tot = (long long)n_rows * SLM_NW * SLM_NTOT;
+        int rc;
+        if ((rc = hs.push(&a.x, &a.ch_stride, n_rows, n_samples, &a.state,
+                          (size_t)n_rows * SLM_STATE_DOUBLES * sizeof(double), fresh)) ||
+            (rc = hs.out(levels, out_stride * SLM_NCOL, ndone * SLM_NCOL, n_rows, &a.levels)) ||
+            (rc = hs.out(totals, tot, tot, 1, &a.totals)))
+            return rc;
+        a.out_stride = ndone;
     }
     slm_kernel<<<(unsigned)((n_rows + SLM_ROWS - 1) / SLM_ROWS), SLM_NW * 32, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 1;
-    if (mem == OMEGA4_MEM_HOST) {
-        if (a.levels) CK(cudaMemcpy2DAsync(levels, out_stride * blk_bytes, a.levels, ndone * blk_bytes, ndone * blk_bytes,
-                                           n_rows, cudaMemcpyDeviceToHost, s));
-        if (a.totals) CK(cudaMemcpyAsync(totals, a.totals, tot_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaMemcpyAsync(state, a.state, st_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
 }
 
 extern "C" int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, const float* levels, int n_rows,
@@ -2589,8 +2625,7 @@ extern "C" int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, cons
                                       float* out) {
     if (!h || !levels || !out || !pct || n_rows < 0 || n_steps < 0 || stride < n_steps)
         return fail(OMEGA4_ERR_INVALID, "bad arguments");
-    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    if (int rc = check_mem(mem)) return rc;
     if (column < 0 || column >= SLM_NCOL) return fail(OMEGA4_ERR_INVALID, "column must be 0 .. 17");
     if (n_pct < 1 || n_pct > SLM_MAX_PCT) return fail(OMEGA4_ERR_INVALID, "n_pct must be 1 .. OMEGA4_SLM_MAX_PCT");
     if (((uintptr_t)levels & 3) || ((uintptr_t)out & 3))
@@ -2607,22 +2642,17 @@ extern "C" int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, cons
     CK(cudaSetDevice(h->device));
     cudaStream_t s = (cudaStream_t)stream;
     a.levels = levels; a.stride = stride; a.n_steps = n_steps; a.column = column; a.n_pct = n_pct; a.out = out;
-    const size_t out_bytes = (size_t)n_rows * n_pct * sizeof(float);
-    int rc;
+    HostStage& hs = h->stage;
     if (mem == OMEGA4_MEM_HOST) {
-        const size_t row_bytes = (size_t)n_steps * SLM_NCOL * sizeof(float);
-        if ((rc = h->h_levels.ensure(n_steps ? (size_t)n_rows * row_bytes : sizeof(float)))) return rc;
-        if ((rc = h->h_out.ensure(out_bytes))) return rc;
-        if (n_steps) CK(cudaMemcpy2DAsync(h->h_levels.p, row_bytes, levels, (size_t)stride * SLM_NCOL * sizeof(float),
-                                          row_bytes, n_rows, cudaMemcpyHostToDevice, s));
-        a.levels = (const float*)h->h_levels.p; a.stride = n_steps; a.out = (float*)h->h_out.p;
+        hs.begin(s);
+        int rc;
+        if ((rc = hs.in(levels, stride * SLM_NCOL, (long long)n_steps * SLM_NCOL, n_rows, &a.levels)) ||
+            (rc = hs.out(out, n_pct, n_pct, n_rows, &a.out)))
+            return rc;
+        a.stride = n_steps;
     }
     slm_percentile_kernel<<<(unsigned)n_rows, SLM_PCT_THREADS, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 1;
-    if (mem == OMEGA4_MEM_HOST) {
-        CK(cudaMemcpyAsync(out, a.out, out_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
 }

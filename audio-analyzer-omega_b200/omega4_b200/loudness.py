@@ -22,58 +22,24 @@ import numpy as np
 
 from . import _native as N
 from . import tables
+from ._blockmeter import BlockMeter, Handle, host_input
+from .tables import check_meter_rate as _check_rate
 
 SUMMARY_KEYS = ("integrated", "lra", "max_momentary", "max_short_term")
 
 
-def _check_rate(sample_rate) -> int:
-    """The sample rate as an int; raises ValueError unless it is an integer multiple of 10 (100 ms sub-blocks) in
-    [8000, 192000].  Below a few kHz the closed-form K-weighting shelf has poles outside the unit circle."""
-    try:
-        fs = int(sample_rate)
-    except (TypeError, ValueError):
-        raise ValueError(f"sample rate {sample_rate!r} must be an integer") from None
-    if fs != sample_rate or fs % 10 or not 8000 <= fs <= 192000:
-        raise ValueError(f"sample rate {sample_rate} must be an integer multiple of 10 in [8000, 192000] "
-                         "(100 ms sub-blocks)")
-    return fs
-
-
-class _Handle:
+class _Handle(Handle):
     """Owns one omega4_loudness object (sample rate, channel weights, K-weighting coefficients)."""
 
     def __init__(self, sample_rate: int, weights: np.ndarray, device: int):
-        lib = N.lib()
-        N.require_device()
-        self.sample_rate, self.sub, self.channels = sample_rate, sample_rate // 10, int(weights.size)
-        if self.channels > N.LOUDNESS_MAX_CH:
-            raise ValueError(f"at most {N.LOUDNESS_MAX_CH} channels per stream, got {self.channels}")
-        self._w = np.ascontiguousarray(weights, dtype=np.float64)
-        self._k = [np.ascontiguousarray(c, dtype=np.float64) for c in tables.bs1770_k_weighting(sample_rate)]
+        if weights.size > N.LOUDNESS_MAX_CH:
+            raise ValueError(f"at most {N.LOUDNESS_MAX_CH} channels per stream, got {weights.size}")
+        w = np.ascontiguousarray(weights, dtype=np.float64)
+        k = [np.ascontiguousarray(c, dtype=np.float64) for c in tables.bs1770_k_weighting(sample_rate)]
         dp = C.POINTER(C.c_double)
-        d = N.LoudnessDesc()
-        d.sample_rate, d.channels, d.sub = sample_rate, self.channels, self.sub
-        d.ch_weights = self._w.ctypes.data_as(dp)
-        d.shelf_b, d.shelf_a, d.hp_b, d.hp_a = (k.ctypes.data_as(dp) for k in self._k)
-        self.ptr = lib.omega4_loudness_create(C.byref(d), int(device))
-        if not self.ptr:
-            raise N.Omega4CudaError(f"omega4_loudness_create failed: {N.last_error()}")
-        self.state_doubles = int(lib.omega4_loudness_state_doubles(self.ptr))
-
-    @property
-    def launches(self) -> int:
-        return int(N.lib().omega4_loudness_launches(self.ptr))
-
-    def close(self):
-        if self.ptr:
-            N.lib().omega4_loudness_destroy(self.ptr)
-            self.ptr = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+        d = N.LoudnessDesc(sample_rate, w.size, w.ctypes.data_as(dp), *(c.ctypes.data_as(dp) for c in k),
+                           sample_rate // 10)
+        super().__init__("loudness", d, device)
 
 
 def _summary_dict(out: np.ndarray, peak_db: np.ndarray) -> Dict[str, np.ndarray]:
@@ -82,37 +48,27 @@ def _summary_dict(out: np.ndarray, peak_db: np.ndarray) -> Dict[str, np.ndarray]
     return d
 
 
-class LoudnessMeter:
+class LoudnessMeter(BlockMeter):
     """Program loudness of ``n_streams`` streams of the same layout, fed tile by tile with device tensors.
 
     ``layout_or_weights``: "mono", "stereo", "5.1" (L R C LFE Ls Rs) or an explicit list of C channel
     weights (7.1 and other layouts).  ``max_seconds`` sizes the device series ``momentary`` / ``short_term``
-    ([n_streams, steps], one step per completed 100 ms sub-block, NaN until the 400 ms / 3 s window fills)."""
+    ([n_streams, steps], one step per completed 100 ms sub-block, NaN until the 400 ms / 3 s window fills).
+    ``launches`` counts two kernels per push and one per summary."""
 
     def __init__(self, sample_rate: int, layout_or_weights: Union[str, Sequence[float]], n_streams: int,
                  max_seconds: float, device: int = 0):
         import torch
-        fs = _check_rate(sample_rate)
         w = tables.bs1770_channel_weights(layout_or_weights)
         if int(n_streams) < 1:
             raise ValueError("n_streams must be >= 1")
-        if not max_seconds > 0:
-            raise ValueError("max_seconds must be > 0")
-        self._h = _Handle(fs, w, device)
-        self.sample_rate, self.sub, self.channels, self.n_streams = fs, fs // 10, int(w.size), int(n_streams)
-        self.capacity = int(np.ceil(float(max_seconds) * 10 - 1e-9))
-        self.dev = torch.device(f"cuda:{device}")
+        self.channels, self.n_streams = int(w.size), int(n_streams)
+        super().__init__(lambda fs, dev: _Handle(fs, w, dev), sample_rate, self.n_streams * self.channels,
+                         self.n_streams, max_seconds, device)
         self._series_m = torch.full((self.n_streams, self.capacity), float("nan"), dtype=torch.float32, device=self.dev)
         self._series_s = torch.full_like(self._series_m, float("nan"))
-        self._state = torch.zeros((self.n_streams, self._h.state_doubles), dtype=torch.float64, device=self.dev)
         self._peak = torch.full((self.n_streams, self.channels), float("-inf"), dtype=torch.float32, device=self.dev)
         self._out = torch.empty((self.n_streams, 4), dtype=torch.float32, device=self.dev)
-        self.samples = 0
-
-    @property
-    def steps(self) -> int:
-        """Completed 100 ms sub-blocks per stream so far."""
-        return self.samples // self.sub
 
     @property
     def momentary(self):
@@ -128,11 +84,6 @@ class LoudnessMeter:
         (-inf for silence and before the first push)."""
         return self._peak
 
-    @property
-    def launches(self) -> int:
-        """Kernels this meter's native object has launched (two per push, one per summary)."""
-        return self._h.launches
-
     def reset(self) -> None:
         """Start every stream anew: the next push ignores the carried state and rewrites the series from step 0;
         the sample peaks read -inf until then."""
@@ -143,27 +94,11 @@ class LoudnessMeter:
         """Continue every stream by ``tile``: float32 CUDA tensor [n_streams * C, n] (rows stream-major,
         unit stride along time, any row stride -- ``StreamBatch.tile_view`` qualifies).  Asynchronous on
         ``stream`` (default: torch's current stream).  Returns the number of steps this push completed."""
-        import torch
-        if not isinstance(tile, torch.Tensor) or not tile.is_cuda:
-            raise ValueError("tile must be a CUDA tensor")
-        if tile.dtype != torch.float32:
-            raise ValueError(f"tile must be float32, got {tile.dtype}")
-        if tile.dim() != 2 or tile.shape[0] != self.n_streams * self.channels:
-            raise ValueError(f"tile must be [{self.n_streams * self.channels}, n], got {tuple(tile.shape)}")
-        if tile.device != self.dev:
-            raise ValueError(f"tile is on {tile.device}, the meter on {self.dev}")
-        n = int(tile.shape[1])
+        n, row_stride, j0, done, s = self._tile(tile, stream)
         if n == 0:
             return 0
-        if tile.stride(1) != 1:
-            raise ValueError("tile rows must be contiguous along time")
-        j0 = self.samples // self.sub
-        done = (self.samples + n) // self.sub - j0
-        if j0 + done > self.capacity:
-            raise ValueError(f"push would exceed max_seconds ({self.capacity} steps); reset() or size the meter larger")
-        s = stream if stream is not None else torch.cuda.current_stream(self.dev).cuda_stream
         rc = N.lib().omega4_loudness_push(
-            self._h.ptr, s, N.MEM_DEVICE, tile.data_ptr(), tile.stride(0), self.n_streams, n,
+            self._h.ptr, s, N.MEM_DEVICE, tile.data_ptr(), row_stride, self.n_streams, n,
             self._state.data_ptr(), 1 if self.samples == 0 else 0, self.capacity,
             self._series_m.data_ptr() + 4 * j0, self._series_s.data_ptr() + 4 * j0, self._peak.data_ptr())
         N.check(rc, "omega4_loudness_push")
@@ -173,16 +108,11 @@ class LoudnessMeter:
     def summary(self, stream=None) -> Dict[str, np.ndarray]:
         """Per stream (numpy arrays): ``integrated`` (LUFS, -inf when no block passes the gates), ``lra`` (LU),
         ``max_momentary``, ``max_short_term`` (NaN while undefined) and ``sample_peak`` [n_streams, C] (dBFS)."""
-        import torch
-        s = stream if stream is not None else torch.cuda.current_stream(self.dev).cuda_stream
-        rc = N.lib().omega4_loudness_summary(self._h.ptr, s, N.MEM_DEVICE, self._series_m.data_ptr(),
-                                             self._series_s.data_ptr(), self.n_streams, self.steps, self.capacity,
-                                             self._out.data_ptr())
+        rc = N.lib().omega4_loudness_summary(self._h.ptr, self._stream(stream), N.MEM_DEVICE,
+                                             self._series_m.data_ptr(), self._series_s.data_ptr(), self.n_streams,
+                                             self.steps, self.capacity, self._out.data_ptr())
         N.check(rc, "omega4_loudness_summary")
         return _summary_dict(self._out.cpu().numpy(), self._peak.cpu().numpy())
-
-    def close(self) -> None:
-        self._h.close()
 
 
 def program_loudness(x: np.ndarray, sample_rate: int, layout: Union[str, Sequence[float]] = "stereo",
@@ -190,17 +120,13 @@ def program_loudness(x: np.ndarray, sample_rate: int, layout: Union[str, Sequenc
     """Host convenience: x float32 [n_streams, C, n] -> the ``LoudnessMeter.summary`` dict plus the
     ``momentary`` / ``short_term`` series [n_streams, n // (sample_rate / 10)] as numpy arrays."""
     fs = _check_rate(sample_rate)
-    x = np.asarray(x)
-    if x.dtype != np.float32:
-        raise ValueError(f"x must be float32, got {x.dtype}")
-    if x.ndim != 3:
-        raise ValueError(f"x must be [n_streams, C, n], got shape {x.shape}")
+    x = host_input(x, 3, "[n_streams, C, n]")
     n_streams, n_ch, n = x.shape
     w = tables.bs1770_channel_weights(layout, n_ch)
     h = _Handle(fs, w, device)
     try:
-        xc = np.ascontiguousarray(x).reshape(n_streams * n_ch, n)
-        steps = n // h.sub
+        xc = x.reshape(n_streams * n_ch, n)
+        steps = n // (fs // 10)
         state = np.zeros((n_streams, h.state_doubles), np.float64)
         mom = np.full((n_streams, steps), np.nan, np.float32)
         sht = np.full_like(mom, np.nan)

@@ -28,6 +28,7 @@ import numpy as np
 
 from . import _native as N
 from . import tables
+from ._blockmeter import BlockMeter, Handle, host_input
 
 WEIGHTINGS = ("A", "C", "Z")
 QUANTITIES = ("eq", "Fmax", "Smax", "F", "S", "peak")
@@ -51,71 +52,35 @@ def _pct(ns: Sequence[float]) -> np.ndarray:
     return p
 
 
-class _Handle:
+class _Handle(Handle):
     """Owns one omega4_slm object (sample rate, weighting coefficients, staging buffers)."""
 
-    def __init__(self, sample_rate, device: int):
-        fs = tables.check_octave_rate(sample_rate)
-        lib = N.lib()
-        N.require_device()
-        self.sample_rate, self.sub = fs, fs // 10
-        self._sos_a = np.ascontiguousarray(tables.iec61672_weighting_sos("A", fs), dtype=np.float64)
-        self._sos_c = np.ascontiguousarray(tables.iec61672_weighting_sos("C", fs), dtype=np.float64)
+    def __init__(self, fs: int, device: int):
+        sa, sc = (np.ascontiguousarray(tables.iec61672_weighting_sos(k, fs), dtype=np.float64) for k in "AC")
         dp = C.POINTER(C.c_double)
-        d = N.SlmDesc(fs, self.sub, self._sos_a.ctypes.data_as(dp), self._sos_c.ctypes.data_as(dp))
-        self.ptr = lib.omega4_slm_create(C.byref(d), int(device))
-        if not self.ptr:
-            raise N.Omega4CudaError(f"omega4_slm_create failed: {N.last_error()}")
-        self.state_doubles = int(lib.omega4_slm_state_doubles(self.ptr))
-
-    @property
-    def launches(self) -> int:
-        return int(N.lib().omega4_slm_launches(self.ptr))
-
-    def close(self):
-        if self.ptr:
-            N.lib().omega4_slm_destroy(self.ptr)
-            self.ptr = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
+        super().__init__("slm", N.SlmDesc(fs, fs // 10, sa.ctypes.data_as(dp), sc.ctypes.data_as(dp)), device)
 
 
-class SoundLevelMeter:
+class SoundLevelMeter(BlockMeter):
     """Sound level meter of ``n_rows`` channel rows, fed tile by tile with device tensors.
 
     ``max_seconds`` sizes the device series ``levels`` ([n_rows, steps, 3, 6], one step per completed 100 ms
     block).  Rows are independent channels.  F and S start from silence, so they read low for the first few
-    time constants (0.125 s and 1 s)."""
+    time constants (0.125 s and 1 s).  ``launches`` counts one kernel per push and one per percentile query."""
 
     WEIGHTINGS = WEIGHTINGS
     QUANTITIES = QUANTITIES
 
     def __init__(self, sample_rate: int, n_rows: int, max_seconds: float, device: int = 0):
         import torch
-        fs = tables.check_octave_rate(sample_rate)
         if int(n_rows) < 1:
             raise ValueError("n_rows must be >= 1")
-        if not max_seconds > 0:
-            raise ValueError("max_seconds must be > 0")
-        self._h = _Handle(fs, device)
-        self.sample_rate, self.sub, self.n_rows = fs, fs // 10, int(n_rows)
-        self.capacity = int(np.ceil(float(max_seconds) * 10 - 1e-9))
-        self.dev = torch.device(f"cuda:{device}")
+        self.n_rows = int(n_rows)
+        super().__init__(_Handle, sample_rate, self.n_rows, self.n_rows, max_seconds, device)
         nw, nq = len(WEIGHTINGS), len(QUANTITIES)
         self._levels = torch.full((self.n_rows, self.capacity, nw, nq), float("nan"), dtype=torch.float32,
                                   device=self.dev)
         self._totals = torch.full((self.n_rows, nw, len(TOTALS)), float("-inf"), dtype=torch.float32, device=self.dev)
-        self._state = torch.zeros((self.n_rows, self._h.state_doubles), dtype=torch.float64, device=self.dev)
-        self.samples = 0
-
-    @property
-    def steps(self) -> int:
-        """Completed 100 ms blocks per row so far."""
-        return self.samples // self.sub
 
     @property
     def levels(self):
@@ -129,11 +94,6 @@ class SoundLevelMeter:
         last reset (an incomplete last block included); -inf before any energy."""
         return self._totals
 
-    @property
-    def launches(self) -> int:
-        """Kernels this meter's native object has launched (one per push, one per percentile query)."""
-        return self._h.launches
-
     def reset(self) -> None:
         """Start every row anew from silence: the next push ignores the carried state and rewrites the series from
         step 0; ``totals`` read -inf until then."""
@@ -144,27 +104,10 @@ class SoundLevelMeter:
         """Continue every row by ``tile``: float32 CUDA tensor [n_rows, n] (unit stride along time, any row
         stride -- ``StreamBatch.tile_view`` qualifies).  Asynchronous on ``stream`` (default: torch's current
         stream).  Returns the number of 100 ms blocks this push completed."""
-        import torch
-        if not isinstance(tile, torch.Tensor) or not tile.is_cuda:
-            raise ValueError("tile must be a CUDA tensor")
-        if tile.dtype != torch.float32:
-            raise ValueError(f"tile must be float32, got {tile.dtype}")
-        if tile.dim() != 2 or tile.shape[0] != self.n_rows:
-            raise ValueError(f"tile must be [{self.n_rows}, n], got {tuple(tile.shape)}")
-        if tile.device != self.dev:
-            raise ValueError(f"tile is on {tile.device}, the meter on {self.dev}")
-        n = int(tile.shape[1])
+        n, row_stride, j0, done, s = self._tile(tile, stream)
         if n == 0:
             return 0
-        if tile.stride(1) != 1:
-            raise ValueError("tile rows must be contiguous along time")
-        j0 = self.samples // self.sub
-        done = (self.samples + n) // self.sub - j0
-        if j0 + done > self.capacity:
-            raise ValueError(f"push would exceed max_seconds ({self.capacity} steps); reset() or size the meter larger")
-        s = stream if stream is not None else torch.cuda.current_stream(self.dev).cuda_stream
         cols = len(WEIGHTINGS) * len(QUANTITIES)
-        row_stride = tile.stride(0) if self.n_rows > 1 else n      # torch gives a single row any stride, even 0
         rc = N.lib().omega4_slm_push(
             self._h.ptr, s, N.MEM_DEVICE, tile.data_ptr(), row_stride, self.n_rows, n, self._state.data_ptr(),
             1 if self.samples == 0 else 0, self.capacity, self._levels.data_ptr() + 4 * j0 * cols,
@@ -183,14 +126,11 @@ class SoundLevelMeter:
         col = _column(weighting, quantity)
         p = _pct(ns)
         out = torch.empty((self.n_rows, p.size), dtype=torch.float32, device=self.dev)
-        s = stream if stream is not None else torch.cuda.current_stream(self.dev).cuda_stream
-        rc = N.lib().omega4_slm_percentiles(self._h.ptr, s, N.MEM_DEVICE, self._levels.data_ptr(), self.n_rows,
-                                            self.steps, self.capacity, col, p.size, p.ctypes.data, out.data_ptr())
+        rc = N.lib().omega4_slm_percentiles(self._h.ptr, self._stream(stream), N.MEM_DEVICE, self._levels.data_ptr(),
+                                            self.n_rows, self.steps, self.capacity, col, p.size, p.ctypes.data,
+                                            out.data_ptr())
         N.check(rc, "omega4_slm_percentiles")
         return out
-
-    def close(self) -> None:
-        self._h.close()
 
 
 def sound_levels(x: np.ndarray, sample_rate: int, percentiles: Sequence[float] = (10, 50, 90),
@@ -198,25 +138,20 @@ def sound_levels(x: np.ndarray, sample_rate: int, percentiles: Sequence[float] =
     """Host convenience: x float32 [n_rows, n] -> numpy ``levels`` [n_rows, n // (sample_rate / 10), 3, 6],
     ``totals`` [n_rows, 3, 4] and ``percentiles`` [n_rows, len(percentiles)], the LAF,N of ``percentiles``
     (LAF sampled at every block end)."""
-    fs = tables.check_octave_rate(sample_rate)
-    x = np.asarray(x)
-    if x.dtype != np.float32:
-        raise ValueError(f"x must be float32, got {x.dtype}")
-    if x.ndim != 2:
-        raise ValueError(f"x must be [n_rows, n], got shape {x.shape}")
+    fs = tables.check_meter_rate(sample_rate)
+    x = host_input(x, 2, "[n_rows, n]")
     p = _pct(percentiles)
     n_rows, n = x.shape
     h = _Handle(fs, device)
     try:
         lib = N.lib()
-        xc = np.ascontiguousarray(x)
-        steps = n // h.sub
+        steps = n // (fs // 10)
         state = np.zeros((n_rows, h.state_doubles), np.float64)
         levels = np.full((n_rows, steps, len(WEIGHTINGS), len(QUANTITIES)), np.nan, np.float32)
         totals = np.full((n_rows, len(WEIGHTINGS), len(TOTALS)), -np.inf, np.float32)
         pct = np.full((n_rows, p.size), np.nan, np.float32)
         if n_rows and n:
-            rc = lib.omega4_slm_push(h.ptr, None, N.MEM_HOST, xc.ctypes.data, n, n_rows, n, state.ctypes.data, 1,
+            rc = lib.omega4_slm_push(h.ptr, None, N.MEM_HOST, x.ctypes.data, n, n_rows, n, state.ctypes.data, 1,
                                      steps, levels.ctypes.data, totals.ctypes.data)
             N.check(rc, "omega4_slm_push")
         if n_rows:

@@ -263,15 +263,17 @@ THIRD_OCTAVE_X = tuple(range(-17, 14))
 THIRD_OCTAVE_ORDER = 3                     # Butterworth prototype order: a 6th-order band-pass, three biquads
 
 
-def check_octave_rate(sample_rate) -> int:
-    """The sample rate as an int; raises ValueError unless it is an integer multiple of 10 in [8000, 192000]
-    (100 ms blocks of fs / 10 samples)."""
+def check_meter_rate(sample_rate) -> int:
+    """The sample rate of the loudness, one-third-octave and sound level meters as an int; raises ValueError unless
+    it is an integer multiple of 10 (100 ms blocks of fs / 10 samples) in [8000, 192000].  Below a few kHz the
+    closed-form K-weighting shelf has poles outside the unit circle."""
     try:
         fs = int(sample_rate)
     except (TypeError, ValueError):
         raise ValueError(f"sample rate {sample_rate!r} must be an integer") from None
     if fs != sample_rate or fs % 10 or not 8000 <= fs <= 192000:
-        raise ValueError(f"sample rate {sample_rate} must be an integer multiple of 10 in [8000, 192000]")
+        raise ValueError(f"sample rate {sample_rate} must be an integer multiple of 10 in [8000, 192000] "
+                         "(100 ms blocks)")
     return fs
 
 
@@ -280,7 +282,7 @@ def third_octave_bands(sample_rate) -> dict:
     edges f_m * 10^(-/+ 1/20); a band is included iff its upper edge f2 < fs / 2 (31 bands at 48 and
     96 kHz, 30 at 44.1 kHz, 23 at 8 kHz).  Returns float64 / int arrays ``x``, ``fm``, ``f1``, ``f2`` and
     the nominal labels ``nominal``."""
-    fs = check_octave_rate(sample_rate)
+    fs = check_meter_rate(sample_rate)
     x = np.array(THIRD_OCTAVE_X)
     fm = 1000.0 * 10.0 ** (0.1 * x)
     f1, f2 = fm * 10.0 ** -0.05, fm * 10.0 ** 0.05
@@ -297,7 +299,7 @@ def third_octave_sos(sample_rate) -> np.ndarray:
     pre-warped as 4 tan(pi Wn / 2), bilinear map z = (4 + s) / (4 - s)), so the coefficients agree with
     scipy's to float64 rounding.  Each conjugate pole pair gets one zero pair (z = 1 and z = -1, numerator
     g * [1, 0, -1]); the three sections share the gain equally.  The gain is 1/sqrt(2) at f1 and f2."""
-    fs = check_octave_rate(sample_rate)
+    fs = check_meter_rate(sample_rate)
     b = third_octave_bands(fs)
     N = THIRD_OCTAVE_ORDER
     proto = -np.exp(1j * np.pi * np.arange(-N + 1, N, 2) / (2 * N))     # left half-plane unit-circle poles
@@ -331,7 +333,7 @@ def iec61672_weighting_sos(kind: str, sample_rate) -> np.ndarray:
     excess poles bring zeros at z = -1.  Sections in scipy's ``zpk2sos`` pairing: the f4 pair with
     g [1, 2, 1], then (A only) the f2 / f3 pair and the f1 pair with g [1, -2, 1]; the sections share the
     gain equally.  The design falls below the analog curve toward Nyquist (DESIGN.md section 4.9)."""
-    fs = check_octave_rate(sample_rate)
+    fs = check_meter_rate(sample_rate)
     f1, f2, f3, f4 = IEC61672_POLE_HZ
     if kind == "A":
         plan = (((f4, f4), 2.0), ((f2, f3), -2.0), ((f1, f1), -2.0))

@@ -300,6 +300,21 @@ int omega4_bars_count(const omega4_bars* bars);
 int omega4_bars_run(omega4_bars* bars, void* stream, int mem, const float* spectrum, int n_ch, int n_hops,
                     float* state, int fresh, float* band_values, float* peak_values);
 
+/* ---- block meters: the push contract of omega4_loudness_push, omega4_octave_push, omega4_slm_push ---- */
+/* The three meters below measure on 100 ms blocks of sub = sample_rate / 10 samples, counted from the stream start,
+ * and a push continues every row of a state array by n_samples samples:
+ *   samples    n_rows rows of float32, row r at samples + r * ch_stride (ch_stride >= n_samples)
+ *   state      doubles, [rows of state][omega4_<meter>_state_doubles], read (unless fresh) and written; every row of
+ *              one state array has received the same number of samples T (each push advances all of them)
+ *   fresh      != 0: start every row anew (T = 0), ignoring the contents of state
+ *   series     [rows of state][out_stride][...] float32, or NULL: column i of row r receives block floor(T / sub) + i.
+ *              A push of n samples after T completes floor((T + n) / sub) - floor(T / sub) blocks, so the caller
+ *              knows the count without a sync.  Blocks at column >= out_stride are not written (in host mode an
+ *              out_stride below the count is an error).
+ *   alignment  samples and every float output float-aligned (no wider alignment is needed), state double-aligned
+ * Tile lengths are arbitrary (no multiple of sub or of 512 needed).  One call at a time per object: it owns its
+ * scratch and OMEGA4_MEM_HOST staging buffers. */
+
 /* ---- ITU-R BS.1770-4 program loudness and EBU Tech 3342 loudness range (extension) ---------- */
 /* Not part of the reference's behaviour: ProfessionalMetering (omega4_analyze's five meters) is not textbook
  * BS.1770 and stays as it is.  This object measures, per stream of C planar channels, the K-weighted
@@ -310,7 +325,7 @@ int omega4_bars_run(omega4_bars* bars, void* stream, int mem, const float* spect
  * at the end of each sub-block j (counted from the stream start), the running sample peak per channel, and on
  * request the integrated loudness (gated at -70 LUFS and 10 LU below) and the loudness range (short-term values
  * gated at -70 and 20 LU below; v[floor(0.95 (n-1) + 0.5)] - v[floor(0.10 (n-1) + 0.5)] of the sorted survivors).
- * DESIGN.md section 4.7.  One call at a time per object (it owns its scratch buffers). */
+ * DESIGN.md section 4.7. */
 #define OMEGA4_LOUDNESS_MAX_CH 32
 typedef struct omega4_loudness omega4_loudness;
 typedef struct omega4_loudness_desc {
@@ -328,22 +343,17 @@ void omega4_loudness_destroy(omega4_loudness* h);
 /* doubles of carried state per stream: 30 + 6 C (sample count, last 29 sub-block energies, per channel the
  * filter state, the partial sub-block's energy and the sample peak) */
 int omega4_loudness_state_doubles(const omega4_loudness* h);
-/* Continue n_streams streams by n_samples samples each:
- *   samples      [n_streams * C] planar rows (stream-major: row s * C + c), row r at samples + r * ch_stride
- *   state        [n_streams][omega4_loudness_state_doubles] read (unless fresh) and written; every stream of one
- *                state array has received the same number of samples T (each push advances all of them)
- *   fresh        != 0: start every stream anew (T = 0), ignoring the contents of state
- *   momentary, short_term  [n_streams][out_stride] float32 LUFS, or NULL: column i of row s receives step
- *                floor(T / sub) + i of stream s.  A push of n samples after T emits
- *                floor((T + n) / sub) - floor(T / sub) steps, so the caller knows the count without a sync.
+/* Continue n_streams streams by n_samples samples each (two kernel launches; the block-meter push contract above):
+ *   samples      [n_streams * C] planar rows (stream-major: row s * C + c)
+ *   state        [n_streams][omega4_loudness_state_doubles]
+ *   momentary, short_term  series [n_streams][out_stride] float32 LUFS, or NULL: a step is a block of stream s
  *   sample_peak  [n_streams][C] float32 20 log10(max |x|) in dBFS over everything pushed since the start
  *                (-inf for silence), or NULL
- * Tile lengths are arbitrary (no multiple of sub or of 512 needed).  Values above -70 LUFS, the integrated loudness
- * and the loudness range agree across tilings to ~1e-6 LU.  Far below the gate they may not: where digital silence
- * follows a signal, a sub-block more than 100 ms into the silence reads either -inf (when the filter restarted from
- * zero over a silent 100 ms warm-up) or a finite value below -120 LUFS (the filter's decaying ringing, when it
- * continued from an earlier sub-block), and where the filter restarts depends on the push boundaries
- * (DESIGN.md section 4.7). */
+ * Values above -70 LUFS, the integrated loudness and the loudness range agree across tilings to ~1e-6 LU.  Far
+ * below the gate they may not: where digital silence follows a signal, a sub-block more than 100 ms into the
+ * silence reads either -inf (when the filter restarted from zero over a silent 100 ms warm-up) or a finite value
+ * below -120 LUFS (the filter's decaying ringing, when it continued from an earlier sub-block), and where the
+ * filter restarts depends on the push boundaries (DESIGN.md section 4.7). */
 int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, const float* samples, long long ch_stride,
                          int n_streams, long long n_samples, double* state, int fresh, long long out_stride,
                          float* momentary, float* short_term, float* sample_peak);
@@ -366,7 +376,7 @@ long long omega4_loudness_launches(const omega4_loudness* h);
  * also keeps Leq = 10 log10(2 sum y^2 / T) over all T samples pushed (an incomplete last block included) and
  * Lmax, the largest completed-block level; both -inf before any energy.  No channel summation, no weighting.
  * The band frequencies follow IEC 61260-1; conformance to its filter class acceptance limits is not claimed.
- * DESIGN.md section 4.8.  One call at a time per object (it owns its staging buffers). */
+ * DESIGN.md section 4.8. */
 #define OMEGA4_OCTAVE_MAX_BANDS 31
 typedef struct omega4_octave omega4_octave;
 typedef struct omega4_octave_desc {
@@ -384,18 +394,11 @@ void omega4_octave_destroy(omega4_octave* h);
 /* doubles of carried state per row: 1 + 9 (n_bands + 1) (the sample count T, then per column the 6 filter values,
  * the partial block's energy, the energy of the completed blocks and the largest block energy) */
 int omega4_octave_state_doubles(const omega4_octave* h);
-/* Continue n_rows channel rows by n_samples samples each (one kernel launch):
- *   samples   [n_rows] rows, row r at samples + r * ch_stride (ch_stride >= n_samples; float alignment suffices)
- *   state     [n_rows][omega4_octave_state_doubles] doubles, read (unless fresh) and written; every row of one
- *             state array has received the same number of samples T
- *   fresh     != 0: start every row anew (T = 0), ignoring the contents of state
- *   levels    [n_rows][out_stride][n_bands + 1] float32 dBFS, or NULL: column i of row r receives block
- *             floor(T / sub) + i.  A push of n samples after T completes floor((T + n) / sub) - floor(T / sub)
- *             blocks, so the caller knows the count without a sync; blocks at column >= out_stride are not written
- *             (in host mode an out_stride below the count is an error).
+/* Continue n_rows channel rows by n_samples samples each (one kernel launch; the block-meter push contract above):
+ *   state     [n_rows][omega4_octave_state_doubles]
+ *   levels    series [n_rows][out_stride][n_bands + 1] float32 dBFS, or NULL
  *   leq, lmax [n_rows][n_bands + 1] float32 dBFS over everything pushed since the start, or NULL
- * Tile lengths are arbitrary: the carried state is exact, so any cut of a stream into pushes gives bit-identical
- * levels, Leq and Lmax. */
+ * The carried state is exact, so any cut of a stream into pushes gives bit-identical levels, Leq and Lmax. */
 int omega4_octave_push(omega4_octave* h, void* stream, int mem, const float* samples, long long ch_stride, int n_rows,
                        long long n_samples, double* state, int fresh, long long out_stride, float* levels, float* leq,
                        float* lmax);
@@ -420,7 +423,7 @@ long long omega4_octave_launches(const omega4_octave* h);
  *   3 LF = v_F at the block's last sample          4 LS = v_S there                      5 Lpeak = 20 log10 max |y_n|
  * Totals per weighting over every sample pushed since the start (an incomplete last block included):
  *   0 Leq = 10 log10(sum e / T)   1 LFmax   2 LSmax   3 Lpeak   (maxima over every pushed sample)
- * DESIGN.md section 4.9.  One call at a time per object (it owns its staging buffers). */
+ * DESIGN.md section 4.9. */
 #define OMEGA4_SLM_WEIGHTINGS 3
 #define OMEGA4_SLM_QUANTITIES 6
 #define OMEGA4_SLM_TOTALS 4
@@ -439,18 +442,11 @@ void omega4_slm_destroy(omega4_slm* h);
 /* doubles of carried state per row: 41 (the sample count T; per weighting the filter values (6, 4, 0), v_F, v_S,
  * the partial block's energy and its maxima of v_F, v_S and e, the completed blocks' energy and their maxima) */
 int omega4_slm_state_doubles(const omega4_slm* h);
-/* Continue n_rows channel rows by n_samples samples each (one kernel launch):
- *   samples   [n_rows] rows, row r at samples + r * ch_stride (ch_stride >= n_samples; float alignment suffices)
- *   state     [n_rows][omega4_slm_state_doubles] doubles, read (unless fresh) and written; every row of one state
- *             array has received the same number of samples T
- *   fresh     != 0: start every row anew (T = 0), ignoring the contents of state
- *   levels    [n_rows][out_stride][3][6] float32 dB (weighting A, C, Z; quantity as above), or NULL: column i of row
- *             r receives block floor(T / sub) + i.  A push of n samples after T completes floor((T + n) / sub) -
- *             floor(T / sub) blocks; blocks at column >= out_stride are not written (in host mode an out_stride
- *             below the count is an error).
+/* Continue n_rows channel rows by n_samples samples each (one kernel launch; the block-meter push contract above):
+ *   state     [n_rows][omega4_slm_state_doubles]
+ *   levels    series [n_rows][out_stride][3][6] float32 dB (weighting A, C, Z; quantity as above), or NULL
  *   totals    [n_rows][3][4] float32 dB over everything pushed since the start, or NULL
- * Tile lengths are arbitrary: the carried state is exact, so any cut of a stream into pushes gives bit-identical
- * levels, totals and state. */
+ * The carried state is exact, so any cut of a stream into pushes gives bit-identical levels, totals and state. */
 int omega4_slm_push(omega4_slm* h, void* stream, int mem, const float* samples, long long ch_stride, int n_rows,
                     long long n_samples, double* state, int fresh, long long out_stride, float* levels, float* totals);
 /* Percentile levels of one series column (one kernel launch): for each row r the first n_steps values
