@@ -301,6 +301,129 @@ static void build_biquad(const double* b, const double* a, int order, KwBiquad* 
 }
 
 // ------------------------------------------------------------------------------------------
+// host side shared by the entry points: device buffers, the device preamble, `mem`, OMEGA4_MEM_HOST staging
+// ------------------------------------------------------------------------------------------
+struct DevBuf {
+    void* p = nullptr;
+    size_t cap = 0;
+    int ensure(size_t bytes) {
+        if (bytes <= cap) return OMEGA4_OK;
+        if (p) cudaFree(p);
+        p = nullptr; cap = 0;
+        CK(cudaMalloc(&p, bytes));
+        cap = bytes;
+        return OMEGA4_OK;
+    }
+    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+};
+
+// a create, or a call without a plan or object: `device` made current
+static int use_device(int device) {
+    if (omega4_device_count() == 0) return fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback");
+    const cudaError_t e = cudaSetDevice(device);
+    if (e != cudaSuccess) return fail(OMEGA4_ERR_CUDA, std::string("cudaSetDevice failed: ") + cudaGetErrorString(e));
+    return OMEGA4_OK;
+}
+
+static int check_mem(int mem) {
+    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
+        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
+    return OMEGA4_OK;
+}
+
+// The arrays of one call.  In OMEGA4_MEM_HOST mode in() and inout() copy host arrays to device buffers, out() gives
+// a device buffer, and finish() copies the outputs and the in/out arrays back and synchronises once; in
+// OMEGA4_MEM_DEVICE mode they hand the caller's pointers through.  table() copies host memory in either mode (the
+// tables the header declares HOST); scratch() is a device buffer the caller never sees.  Sizes and pitches are in
+// elements.  An object's stage keeps its buffers between calls (they only grow); a stage made for one call frees
+// them when it goes out of scope, so its finish() also waits for device-mode work that reads them.
+struct HostStage {
+    DevBuf buf[OMEGA4_MAX_RES + 1];   // one per array a call stages; omega4_combine stages the most
+    struct Back { void* dst; const void* src; size_t dpitch, width, rows; } back[4];     // bytes
+    int nbuf = 0, nback = 0;
+    cudaStream_t s = nullptr;
+    bool host = false, allocated = false;
+    const bool per_call;
+
+    HostStage() : per_call(false) {}
+    HostStage(cudaStream_t stream, int mem) : per_call(true) { begin(stream, mem); }
+    ~HostStage() { if (per_call) release(); }
+    HostStage(const HostStage&) = delete;
+    HostStage& operator=(const HostStage&) = delete;
+
+    void begin(cudaStream_t stream, int mem) {
+        s = stream; host = mem == OMEGA4_MEM_HOST; nbuf = nback = 0; allocated = false;
+    }
+
+    // rows x width bytes between two pitched arrays; one plain copy when both are dense
+    cudaError_t copy(void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t rows,
+                     cudaMemcpyKind kind) {
+        if (dpitch == width && spitch == width) return cudaMemcpyAsync(dst, src, width * rows, kind, s);
+        return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, s);
+    }
+
+    template <class T> int scratch(long long n, T** dev) {
+        DevBuf& b = buf[nbuf++];
+        if (int rc = b.ensure((size_t)std::max(n, 1LL) * sizeof(T))) return rc;
+        allocated = true;
+        *dev = (T*)b.p;
+        return OMEGA4_OK;
+    }
+
+    // rows x width elements of host memory at src (row pitch spitch) -> a dense device copy; nullptr for a null src
+    template <class T> int table(const T* src, long long spitch, long long width, long long rows, const T** dev) {
+        *dev = nullptr;
+        if (!src) return OMEGA4_OK;
+        T* d;
+        if (int rc = scratch(width * rows, &d)) return rc;
+        if (width * rows)
+            CK(copy(d, width * sizeof(T), src, spitch * sizeof(T), width * sizeof(T), rows, cudaMemcpyHostToDevice));
+        *dev = d;
+        return OMEGA4_OK;
+    }
+    template <class T> int table(const T* src, long long n, const T** dev) { return table(src, n, n, 1, dev); }
+
+    template <class T> int in(const T* src, long long spitch, long long width, long long rows, const T** dev) {
+        if (host) return table(src, spitch, width, rows, dev);
+        *dev = src;
+        return OMEGA4_OK;
+    }
+    template <class T> int in(const T* src, long long n, const T** dev) { return in(src, n, n, 1, dev); }
+
+    // rows x width elements for dst (row pitch dpitch); in host mode nullptr when dst is null or there is nothing
+    // to write
+    template <class T> int out(T* dst, long long dpitch, long long width, long long rows, T** dev) {
+        *dev = host ? nullptr : dst;
+        if (!host || !dst || width * rows == 0) return OMEGA4_OK;
+        if (int rc = scratch(width * rows, dev)) return rc;
+        back[nback++] = {dst, *dev, dpitch * sizeof(T), width * sizeof(T), (size_t)rows};
+        return OMEGA4_OK;
+    }
+    template <class T> int out(T* dst, long long n, T** dev) { return out(dst, n, n, 1, dev); }
+
+    // n elements the call reads (unless fresh) and writes
+    template <class T> int inout(T* p, long long n, int fresh, T** dev) {
+        *dev = p;
+        if (!host || !p) return OMEGA4_OK;
+        if (int rc = scratch(n, dev)) return rc;
+        if (!fresh) CK(cudaMemcpyAsync(*dev, p, n * sizeof(T), cudaMemcpyHostToDevice, s));
+        back[nback++] = {p, *dev, n * sizeof(T), n * sizeof(T), 1};
+        return OMEGA4_OK;
+    }
+
+    int finish() {
+        for (int i = 0; i < nback; ++i) {
+            const Back& c = back[i];
+            CK(copy(c.dst, c.dpitch, c.src, c.width, c.width, c.rows, cudaMemcpyDeviceToHost));
+        }
+        if (host || (per_call && allocated)) CK(cudaStreamSynchronize(s));
+        return OMEGA4_OK;
+    }
+
+    void release() { for (DevBuf& b : buf) b.release(); }
+};
+
+// ------------------------------------------------------------------------------------------
 // plan
 // ------------------------------------------------------------------------------------------
 struct ResInfo {
@@ -348,20 +471,6 @@ struct SparseSet {
     }
 };
 
-struct DevBuf {
-    void* p = nullptr;
-    size_t cap = 0;
-    int ensure(size_t bytes) {
-        if (bytes <= cap) return OMEGA4_OK;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        CK(cudaMalloc(&p, bytes));
-        cap = bytes;
-        return OMEGA4_OK;
-    }
-    void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
-
 // ------------------------------------------------------------------------------------------
 // application post-processing object (omega4_bars_*); also used fused behind the combine by omega4_analyze_io
 // ------------------------------------------------------------------------------------------
@@ -369,7 +478,8 @@ struct omega4_bars {
     int device = 0, T = 0, n_valid = 0, p_lo = 0, normalize_max = 0;
     float p_frac = 0.f, scale = 0.8f;
     int* bands = nullptr; float* gain = nullptr; float* sf = nullptr; float* sfc = nullptr;
-    DevBuf h_spec, h_out, h_peak, h_state, state_in;
+    DevBuf state_in;
+    HostStage stage;
 };
 
 // spectrum [n_ch][n_hops][T] (device) -> band values (+ unsmoothed peaks) on stream s; state (device) carries the
@@ -454,7 +564,8 @@ struct omega4_plan {
     SparseSet set_tc;             // 3xTF32 tcgen05 GEMM: up to 512 columns
     bool tensor_default = true;   // OMEGA4_TENSOR=0 makes the CUDA-core GEMM the default
     DevBuf scratch_lufs, scratch_tp, scratch_mag[OMEGA4_MAX_RES], scratch_q, scratch_f32, scratch_comb, scratch_bstate, scratch_inv;
-    DevBuf h_in, h_comb, h_meters, h_state, h_mag[OMEGA4_MAX_RES], h_f64a, h_f64b, h_f64c;
+    DevBuf scratch_state;         // meter state of a device-mode analysis without one
+    HostStage stage;              // omega4_combine, omega4_meter_frames, omega4_meter_stats
     // host-buffer mode: channel chunks are pipelined over N_SLOTS private streams / buffer sets so
     // that H2D of chunk i+1, the kernels of chunk i and D2H of chunk i-1 overlap
     struct Slot {
@@ -924,15 +1035,14 @@ extern "C" void omega4_plan_destroy(omega4_plan* p) {
     for (int r = 0; r < OMEGA4_MAX_RES; ++r) {
         ResInfo& ri = p->res[r];
         cudaFree(ri.window); cudaFree(ri.binw); cudaFree(ri.tb_idx); cudaFree(ri.tb_lo); cudaFree(ri.tb_frac);
-        p->scratch_mag[r].release(); p->h_mag[r].release();
+        p->scratch_mag[r].release();
     }
     cudaFree(p->csr_ptr); cudaFree(p->csr_res); cudaFree(p->csr_lo); cudaFree(p->csr_frac);
     cudaFree(p->hann64); cudaFree(p->hann32); cudaFree(p->tp_rot); cudaFree(p->tp_rot_h);
     p->scratch_lufs.release(); p->scratch_tp.release(); p->scratch_q.release(); p->scratch_f32.release(); p->scratch_inv.release();
-    p->scratch_comb.release(); p->scratch_bstate.release();
+    p->scratch_comb.release(); p->scratch_bstate.release(); p->scratch_state.release();
     p->set_cc.release(); p->set_tc.release();
-    p->h_in.release(); p->h_comb.release(); p->h_meters.release(); p->h_state.release();
-    p->h_f64a.release(); p->h_f64b.release(); p->h_f64c.release();
+    p->stage.release();
     for (auto& sl : p->slots) {
         sl.in.release(); sl.comb.release(); sl.met.release(); sl.lufs.release(); sl.tp.release(); sl.state.release();
         sl.q.release(); sl.in16.release(); sl.sc.release();
@@ -1134,9 +1244,9 @@ static int analyze_device(omega4_plan* p, cudaStream_t s, const float* x, long l
             st.gate = p->gate; st.out = meters;
             st.fresh = (state == nullptr) || (flags & OMEGA4_FLAG_FRESH_METERS) ? 1 : 0;
             if (!state) {
-                int rc = p->h_state.ensure((size_t)n_ch * ST_STATE * sizeof(double));
+                int rc = p->scratch_state.ensure((size_t)n_ch * ST_STATE * sizeof(double));
                 if (rc) return rc;
-                state = (double*)p->h_state.p;
+                state = (double*)p->scratch_state.p;
             }
             st.state = state;
             Bracket b(p, ss, timing, "meter_stats");
@@ -1721,38 +1831,25 @@ extern "C" int omega4_meter_update(omega4_plan* p, const double* frame, double* 
 extern "C" int omega4_combine(omega4_plan* p, void* stream, int mem, const float* const* magnitudes, int n_rows,
                               float* combined) {
     if (!p || !magnitudes || !combined || n_rows < 0) return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_rows == 0) return OMEGA4_OK;
     CK(cudaSetDevice(p->device));
-    cudaStream_t s = (cudaStream_t)stream;
+    HostStage& hs = p->stage;
+    hs.begin((cudaStream_t)stream, mem);
     CombineArgs c;
     memset(&c, 0, sizeof c);
-    float* d_out = combined;
-    if (mem == OMEGA4_MEM_HOST) {
-        for (int r = 0; r < p->n_res; ++r)
-            if (magnitudes[r]) {
-                const size_t bytes = (size_t)n_rows * p->res[r].bins * sizeof(float);
-                int rc = p->h_mag[r].ensure(bytes); if (rc) return rc;
-                CK(cudaMemcpyAsync(p->h_mag[r].p, magnitudes[r], bytes, cudaMemcpyHostToDevice, s));
-                c.mag[r] = (const float*)p->h_mag[r].p;
-            }
-        int rc = p->h_comb.ensure((size_t)n_rows * p->T * sizeof(float)); if (rc) return rc;
-        d_out = (float*)p->h_comb.p;
-    } else {
-        for (int r = 0; r < p->n_res; ++r) c.mag[r] = magnitudes[r];
+    for (int r = 0; r < p->n_res; ++r) {
+        if (int rc = hs.in(magnitudes[r], (long long)n_rows * p->res[r].bins, &c.mag[r])) return rc;
+        c.bins[r] = p->res[r].bins; c.first_frame[r] = 0; c.weight[r] = p->res[r].weight;
     }
-    for (int r = 0; r < p->n_res; ++r) { c.bins[r] = p->res[r].bins; c.first_frame[r] = 0; c.weight[r] = p->res[r].weight; }
     c.n_hops = 0; c.n_rows = n_rows; c.T = p->T;
     c.csr_ptr = p->csr_ptr; c.csr_res = p->csr_res; c.csr_lo = p->csr_lo; c.csr_frac = p->csr_frac;
-    c.out = d_out;
     const long long total = (long long)n_rows * p->T;
+    if (int rc = hs.out(combined, total, &c.out)) return rc;
     p->launches++;
-    combine_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(c);
+    combine_kernel<<<(unsigned)((total + 255) / 256), 256, 0, hs.s>>>(c);
     CK(cudaGetLastError());
-    if (mem == OMEGA4_MEM_HOST) {
-        CK(cudaMemcpyAsync(combined, d_out, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    return hs.finish();
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1761,25 +1858,21 @@ extern "C" int omega4_combine(omega4_plan* p, void* stream, int mem, const float
 extern "C" int omega4_meter_frames(omega4_plan* p, void* stream, int mem, const double* frames, int n_frames,
                                    double* lufs_inst, double* tp_db, double* weighted) {
     if (!p || !frames || n_frames < 0) return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_frames == 0) return OMEGA4_OK;
     CK(cudaSetDevice(p->device));
-    cudaStream_t s = (cudaStream_t)stream;
+    if (mem == OMEGA4_MEM_DEVICE && ((uintptr_t)frames & 15) != 0) return fail(OMEGA4_ERR_INVALID, "frames must be 16-byte aligned");
     const int W = p->W;
-    const double* d_fr = frames; double* d_l = lufs_inst; double* d_t = tp_db; double* d_w = weighted;
-    DevBuf tmp_w;
-    if (mem == OMEGA4_MEM_HOST) {
-        int rc = p->h_f64a.ensure((size_t)n_frames * W * sizeof(double)); if (rc) return rc;
-        CK(cudaMemcpyAsync(p->h_f64a.p, frames, (size_t)n_frames * W * sizeof(double), cudaMemcpyHostToDevice, s));
-        d_fr = (const double*)p->h_f64a.p;
-        rc = p->h_f64b.ensure((size_t)n_frames * 2 * sizeof(double)); if (rc) return rc;
-        d_l = (double*)p->h_f64b.p; d_t = d_l + n_frames;
-        if (weighted) { rc = tmp_w.ensure((size_t)n_frames * W * sizeof(double)); if (rc) return rc; d_w = (double*)tmp_w.p; }
-    } else if (((uintptr_t)frames & 15) != 0) {
-        return fail(OMEGA4_ERR_INVALID, "frames must be 16-byte aligned");
-    }
-    int rc = OMEGA4_OK;
+    HostStage& hs = p->stage;
+    hs.begin((cudaStream_t)stream, mem);
+    const cudaStream_t s = hs.s;
+    const double* d_fr; double* d_l; double* d_t; double* d_w;
+    int rc;
+    if ((rc = hs.in(frames, (long long)n_frames * W, &d_fr)) || (rc = hs.out(lufs_inst, n_frames, &d_l)) ||
+        (rc = hs.out(tp_db, n_frames, &d_t)) || (rc = hs.out(weighted, (long long)n_frames * W, &d_w)))
+        return rc;
     if (lufs_inst || weighted) {
-        if (!d_l || (mem == OMEGA4_MEM_DEVICE && !lufs_inst)) { rc = p->scratch_lufs.ensure((size_t)n_frames * sizeof(double)); if (rc) { tmp_w.release(); return rc; } d_l = (double*)p->scratch_lufs.p; }
+        if (!lufs_inst && (rc = hs.scratch(n_frames, &d_l))) return rc;      // the kernel always writes LUFS
         KweightArgs k;
         memset(&k, 0, sizeof k);
         k.x = d_fr; k.x_is_f64 = 1; k.ch_stride = 0; k.frame_stride = W; k.frame_off0 = 0;
@@ -1787,8 +1880,7 @@ extern "C" int omega4_meter_frames(omega4_plan* p, void* stream, int mem, const 
         k.hann = nullptr; k.lufs_out = d_l; k.weighted_out = d_w;
         fill_weighting(p, &k);
         p->launches++;
-        rc = launch_kweight(k, s);
-        if (rc) { tmp_w.release(); return rc; }
+        if ((rc = launch_kweight(k, s))) return rc;
     }
     if (tp_db) {
         TruePeakArgs t;
@@ -1799,57 +1891,32 @@ extern "C" int omega4_meter_frames(omega4_plan* p, void* stream, int mem, const 
         fill_truepeak_steps(&t);
         t.tp_out = d_t;
         p->launches++;
-        rc = launch_truepeak(t, s);
-        if (rc) { tmp_w.release(); return rc; }
+        if ((rc = launch_truepeak(t, s))) return rc;
     }
-    if (mem == OMEGA4_MEM_HOST) {
-        cudaError_t e = cudaSuccess;
-        if (lufs_inst) e = cudaMemcpyAsync(lufs_inst, d_l, (size_t)n_frames * sizeof(double), cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess && tp_db) e = cudaMemcpyAsync(tp_db, d_t, (size_t)n_frames * sizeof(double), cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess && weighted) e = cudaMemcpyAsync(weighted, d_w, (size_t)n_frames * W * sizeof(double), cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        tmp_w.release();
-        if (e != cudaSuccess) return fail(OMEGA4_ERR_CUDA, std::string("meter_frames copy back failed: ") + cudaGetErrorString(e));
-    }
-    return OMEGA4_OK;
+    return hs.finish();
 }
 
 extern "C" int omega4_meter_stats(omega4_plan* p, void* stream, int mem, const double* lufs_inst, const double* tp_db,
                                   int n_ch, int n_frames, int first_frame, double* state, float* meters, int fresh) {
     if (!p || !lufs_inst || !tp_db || !meters || n_ch < 0 || n_frames < 0) return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_ch == 0 || n_frames == 0) return OMEGA4_OK;
     CK(cudaSetDevice(p->device));
-    cudaStream_t s = (cudaStream_t)stream;
+    HostStage& hs = p->stage;
+    hs.begin((cudaStream_t)stream, mem);
     StatsArgs st;
     memset(&st, 0, sizeof st);
-    const size_t rows = (size_t)n_ch * n_frames;
-    st.n_ch = n_ch; st.n_frames = n_frames; st.first_frame = first_frame; st.gate = p->gate; st.fresh = fresh ? 1 : 0;
-    if (mem == OMEGA4_MEM_HOST) {
-        int rc = p->h_f64a.ensure(rows * 2 * sizeof(double)); if (rc) return rc;
-        double* d = (double*)p->h_f64a.p;
-        CK(cudaMemcpyAsync(d, lufs_inst, rows * sizeof(double), cudaMemcpyHostToDevice, s));
-        CK(cudaMemcpyAsync(d + rows, tp_db, rows * sizeof(double), cudaMemcpyHostToDevice, s));
-        st.lufs = d; st.tp = d + rows;
-        rc = p->h_f64c.ensure((size_t)n_ch * ST_STATE * sizeof(double)); if (rc) return rc;
-        st.state = (double*)p->h_f64c.p;
-        if (state && !fresh) CK(cudaMemcpyAsync(st.state, state, (size_t)n_ch * ST_STATE * sizeof(double), cudaMemcpyHostToDevice, s));
-        else st.fresh = 1;
-        rc = p->h_meters.ensure(rows * 5 * sizeof(float)); if (rc) return rc;
-        st.out = (float*)p->h_meters.p;
-    } else {
-        st.lufs = lufs_inst; st.tp = tp_db; st.out = meters;
-        if (state) st.state = state;
-        else { int rc = p->h_state.ensure((size_t)n_ch * ST_STATE * sizeof(double)); if (rc) return rc; st.state = (double*)p->h_state.p; st.fresh = 1; }
-    }
+    const long long rows = (long long)n_ch * n_frames, st_n = (long long)n_ch * ST_STATE;
+    st.n_ch = n_ch; st.n_frames = n_frames; st.first_frame = first_frame; st.gate = p->gate;
+    st.fresh = (fresh || !state) ? 1 : 0;
+    int rc;
+    if ((rc = hs.in(lufs_inst, rows, &st.lufs)) || (rc = hs.in(tp_db, rows, &st.tp)) ||
+        (rc = hs.out(meters, rows * 5, &st.out)) ||
+        (rc = state ? hs.inout(state, st_n, st.fresh, &st.state) : hs.scratch(st_n, &st.state)))
+        return rc;
     p->launches++;
-    int rc = launch_stats(st, s);
-    if (rc) return rc;
-    if (mem == OMEGA4_MEM_HOST) {
-        CK(cudaMemcpyAsync(meters, st.out, rows * 5 * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (state) CK(cudaMemcpyAsync(state, st.state, (size_t)n_ch * ST_STATE * sizeof(double), cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    if ((rc = launch_stats(st, hs.s))) return rc;
+    return hs.finish();
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1858,88 +1925,50 @@ extern "C" int omega4_meter_stats(omega4_plan* p, void* stream, int mem, const d
 extern "C" int omega4_rfft_batch(int device, void* stream, int mem, const float* frames, int batch, int n,
                                  const float* window, float* magnitude, float* complex_out) {
     if (!frames || batch < 0 || (!magnitude && !complex_out)) return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (!is_pow2(n) || n < 512 || n > 32768) return fail(OMEGA4_ERR_UNSUPPORTED, "fft size must be a power of two in 512 .. 32768");
     if (batch == 0) return OMEGA4_OK;
-    if (omega4_device_count() == 0) return fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback");
-    CK(cudaSetDevice(device));
-    cudaStream_t s = (cudaStream_t)stream;
+    if (int rc = use_device(device)) return rc;
     const int log2m = ilog2(n) - 1, bins = n / 2 + 1;
     Twiddles tw;
     int rc = get_twiddles(device, log2m, &tw);
     if (rc) return rc;
-    float* d_win = nullptr; float* d_in = nullptr; float* d_mag = nullptr; float2* d_c = nullptr;
-    std::vector<void*> to_free;
-    auto cleanup = [&]() { for (void* q : to_free) cudaFree(q); };
-#define CKF(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { cleanup(); return fail(OMEGA4_ERR_CUDA, std::string(#expr " failed: ") + cudaGetErrorString(e__)); } } while (0)
-    if (window) {
-        CKF(cudaMalloc(&d_win, (size_t)n * sizeof(float))); to_free.push_back(d_win);
-        CKF(cudaMemcpyAsync(d_win, window, (size_t)n * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
-    if (mem == OMEGA4_MEM_HOST) {
-        CKF(cudaMalloc(&d_in, (size_t)batch * n * sizeof(float))); to_free.push_back(d_in);
-        CKF(cudaMemcpyAsync(d_in, frames, (size_t)batch * n * sizeof(float), cudaMemcpyHostToDevice, s));
-        if (magnitude) { CKF(cudaMalloc(&d_mag, (size_t)batch * bins * sizeof(float))); to_free.push_back(d_mag); }
-        if (complex_out) { CKF(cudaMalloc(&d_c, (size_t)batch * bins * sizeof(float2))); to_free.push_back(d_c); }
-    } else {
-        if (((uintptr_t)frames & 15) != 0) { cleanup(); return fail(OMEGA4_ERR_INVALID, "frames must be 16-byte aligned"); }
-        d_in = const_cast<float*>(frames); d_mag = magnitude; d_c = reinterpret_cast<float2*>(complex_out);
-    }
+    if (mem == OMEGA4_MEM_DEVICE && ((uintptr_t)frames & 15) != 0) return fail(OMEGA4_ERR_INVALID, "frames must be 16-byte aligned");
+    HostStage hs((cudaStream_t)stream, mem);
     MultiresArgs a;
     memset(&a, 0, sizeof a);
-    a.x = d_in; a.ch_stride = 0; a.frame_stride = n; a.frame_off0 = 0;
-    a.n_ch = 1; a.n_frames = batch; a.first_frame = 0;
+    if ((rc = hs.table(window, n, &a.window)) || (rc = hs.in(frames, (long long)batch * n, &a.x)) ||
+        (rc = hs.out(magnitude, (long long)batch * bins, &a.mag_out)) ||
+        (rc = hs.out(reinterpret_cast<float2*>(complex_out), (long long)batch * bins, &a.cplx_out)))
+        return rc;
+    a.frame_stride = n; a.n_ch = 1; a.n_frames = batch;
     a.rounds = default_rounds(batch, (1 << log2m) >= 4096 ? 1 : 4096 >> log2m);
-    a.window = d_win; a.binw = nullptr; a.twM = tw.twM; a.twN = tw.twN;
-    a.mag_out = d_mag; a.cplx_out = d_c; a.comb_out = nullptr; a.T = 0; a.n_tb = 0; a.need_lo = 0; a.need_cnt = 0;
-    rc = launch_multires(log2m, a, s);
-    if (rc) { cleanup(); return rc; }
-    if (mem == OMEGA4_MEM_HOST) {
-        if (magnitude) CKF(cudaMemcpyAsync(magnitude, d_mag, (size_t)batch * bins * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (complex_out) CKF(cudaMemcpyAsync(complex_out, d_c, (size_t)batch * bins * sizeof(float2), cudaMemcpyDeviceToHost, s));
-    }
-    if (!to_free.empty()) CKF(cudaStreamSynchronize(s));
-    cleanup();
-#undef CKF
-    return OMEGA4_OK;
+    a.twM = tw.twM; a.twN = tw.twN;
+    if ((rc = launch_multires(log2m, a, hs.s))) return rc;
+    return hs.finish();
 }
 
 extern "C" int omega4_band_map(int device, void* stream, int mem, const float* spectrum, int n_rows, int len,
                                const int* bands, int n_bars, const float* comp, float* bars_out, int db) {
     if (!spectrum || !bands || !bars_out || n_rows < 0 || len <= 0 || n_bars <= 0) return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_rows == 0) return OMEGA4_OK;
-    if (omega4_device_count() == 0) return fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback");
-    CK(cudaSetDevice(device));
-    cudaStream_t s = (cudaStream_t)stream;
+    if (int rc = use_device(device)) return rc;
     int n_valid = n_bars;
     for (int b = 0; b < n_bars; ++b) {
         if (bands[2 * b] < 0 || bands[2 * b + 1] < bands[2 * b]) return fail(OMEGA4_ERR_INVALID, "bad band table");
         if (bands[2 * b + 1] > len) { n_valid = b; break; }        // freq_mapper.py:188-189 `break`
     }
-    std::vector<void*> to_free;
-    auto cleanup = [&]() { for (void* q : to_free) cudaFree(q); };
-#define CKF(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { cleanup(); return fail(OMEGA4_ERR_CUDA, std::string(#expr " failed: ") + cudaGetErrorString(e__)); } } while (0)
-    int* d_bands = nullptr; float* d_comp = nullptr; const float* d_spec = spectrum; float* d_out = bars_out;
-    CKF(cudaMalloc(&d_bands, (size_t)n_bars * 2 * sizeof(int))); to_free.push_back(d_bands);
-    CKF(cudaMemcpyAsync(d_bands, bands, (size_t)n_bars * 2 * sizeof(int), cudaMemcpyHostToDevice, s));
-    if (comp) {
-        CKF(cudaMalloc(&d_comp, (size_t)len * sizeof(float))); to_free.push_back(d_comp);
-        CKF(cudaMemcpyAsync(d_comp, comp, (size_t)len * sizeof(float), cudaMemcpyHostToDevice, s));
-    }
-    if (mem == OMEGA4_MEM_HOST) {
-        float* t = nullptr;
-        CKF(cudaMalloc(&t, (size_t)n_rows * len * sizeof(float))); to_free.push_back(t);
-        CKF(cudaMemcpyAsync(t, spectrum, (size_t)n_rows * len * sizeof(float), cudaMemcpyHostToDevice, s));
-        d_spec = t;
-        CKF(cudaMalloc(&d_out, (size_t)n_rows * n_bars * sizeof(float))); to_free.push_back(d_out);
-    }
     const long long total = (long long)n_rows * n_bars;
-    band_map_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(d_spec, n_rows, len, d_bands, n_bars, n_valid, d_comp, d_out, db);
-    CKF(cudaGetLastError());
-    if (mem == OMEGA4_MEM_HOST) CKF(cudaMemcpyAsync(bars_out, d_out, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost, s));
-    CKF(cudaStreamSynchronize(s));
-    cleanup();
-#undef CKF
-    return OMEGA4_OK;
+    HostStage hs((cudaStream_t)stream, mem);
+    const int* d_bands; const float* d_comp; const float* d_spec; float* d_out;
+    int rc;
+    if ((rc = hs.table(bands, 2LL * n_bars, &d_bands)) || (rc = hs.table(comp, len, &d_comp)) ||
+        (rc = hs.in(spectrum, (long long)n_rows * len, &d_spec)) || (rc = hs.out(bars_out, total, &d_out)))
+        return rc;
+    band_map_kernel<<<(unsigned)((total + 255) / 256), 256, 0, hs.s>>>(d_spec, n_rows, len, d_bands, n_bars, n_valid, d_comp, d_out, db);
+    CK(cudaGetLastError());
+    return hs.finish();
 }
 
 extern "C" int omega4_waterfall(int device, void* stream, int mem, const float* spectra, int n_ch, int n_rows, int len,
@@ -1948,59 +1977,32 @@ extern "C" int omega4_waterfall(int device, void* stream, int mem, const float* 
     if (!spectra || n_ch < 0 || n_rows < 0 || len <= 0 || lo < 0 || hi <= lo || hi > len || (db_form != 0 && db_form != 1) ||
         (!db_out && !norm_out && !rowstat_out))
         return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_ch == 0 || n_rows == 0) return OMEGA4_OK;
     if ((long long)n_ch * n_rows > 2147483647LL) return fail(OMEGA4_ERR_INVALID, "too many rows for one waterfall call");
-    if (omega4_device_count() == 0) return fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback");
-    CK(cudaSetDevice(device));
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t rows = (size_t)n_ch * n_rows, n = (size_t)(hi - lo);
-    std::vector<void*> to_free;
-    auto cleanup = [&]() { for (void* q : to_free) cudaFree(q); };
-#define CKF(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { cleanup(); return fail(OMEGA4_ERR_CUDA, std::string(#expr " failed: ") + cudaGetErrorString(e__)); } } while (0)
+    if (int rc = use_device(device)) return rc;
+    const long long rows = (long long)n_ch * n_rows, n = hi - lo;
     WaterfallArgs a;
     memset(&a, 0, sizeof a);
     a.n_ch = n_ch; a.n_rows = n_rows; a.len = len; a.lo = lo; a.hi = hi; a.db_form = db_form; a.auto_gain = auto_gain ? 1 : 0;
     a.gain_adjustment = gain_adjustment;
-    const size_t st_bytes = (size_t)n_ch * WF_STATE * sizeof(float);
-    if (mem == OMEGA4_MEM_HOST) {
-        float* t = nullptr;
-        CKF(cudaMalloc(&t, rows * len * sizeof(float))); to_free.push_back(t);
-        CKF(cudaMemcpyAsync(t, spectra, rows * len * sizeof(float), cudaMemcpyHostToDevice, s));
-        a.spec = t;
-        if (db_out) { CKF(cudaMalloc(&a.db_out, rows * n * sizeof(float))); to_free.push_back(a.db_out); }
-        if (norm_out) { CKF(cudaMalloc(&a.norm_out, rows * n * sizeof(float))); to_free.push_back(a.norm_out); }
-        if (state) {
-            float* d_st = nullptr;
-            CKF(cudaMalloc(&d_st, st_bytes)); to_free.push_back(d_st);
-            if (!fresh) { CKF(cudaMemcpyAsync(d_st, state, st_bytes, cudaMemcpyHostToDevice, s)); a.state_in = d_st; }
-            a.state_out = d_st;
-        }
-    } else if (mem == OMEGA4_MEM_DEVICE) {
-        a.spec = spectra; a.db_out = db_out; a.norm_out = norm_out;
-        a.state_in = (state && !fresh) ? state : nullptr; a.state_out = state;
-    } else {
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
-    }
-    if (mem == OMEGA4_MEM_DEVICE && rowstat_out) a.rowstat = rowstat_out;
-    else { CKF(cudaMalloc(&a.rowstat, rows * 4 * sizeof(float))); to_free.push_back(a.rowstat); }
+    HostStage hs((cudaStream_t)stream, mem);
+    int rc;
+    if ((rc = hs.in(spectra, rows * len, &a.spec)) || (rc = hs.out(db_out, rows * n, &a.db_out)) ||
+        (rc = hs.out(norm_out, rows * n, &a.norm_out)) || (rc = hs.inout(state, (long long)n_ch * WF_STATE, fresh, &a.state_out)) ||
+        (rc = rowstat_out ? hs.out(rowstat_out, rows * 4, &a.rowstat) : hs.scratch(rows * 4, &a.rowstat)))
+        return rc;
+    if (!fresh) a.state_in = a.state_out;
+    const cudaStream_t s = hs.s;
     waterfall_db_kernel<<<(unsigned)rows, 256, 0, s>>>(a);
-    CKF(cudaGetLastError());
+    CK(cudaGetLastError());
     waterfall_norm_kernel<<<(unsigned)rows, 256, 0, s>>>(a);
-    CKF(cudaGetLastError());
+    CK(cudaGetLastError());
     if (a.state_out) {
         waterfall_state_kernel<<<(unsigned)((n_ch + 127) / 128), 128, 0, s>>>(a);
-        CKF(cudaGetLastError());
+        CK(cudaGetLastError());
     }
-    if (mem == OMEGA4_MEM_HOST) {
-        if (db_out) CKF(cudaMemcpyAsync(db_out, a.db_out, rows * n * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (norm_out) CKF(cudaMemcpyAsync(norm_out, a.norm_out, rows * n * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (rowstat_out) CKF(cudaMemcpyAsync(rowstat_out, a.rowstat, rows * 4 * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (state) CKF(cudaMemcpyAsync(state, a.state_out, st_bytes, cudaMemcpyDeviceToHost, s));
-    }
-    if (!to_free.empty()) CKF(cudaStreamSynchronize(s));
-    cleanup();
-#undef CKF
-    return OMEGA4_OK;
+    return hs.finish();
 }
 
 extern "C" int omega4_plan_set_gate_threshold(omega4_plan* p, double gate_threshold) {
@@ -2015,47 +2017,23 @@ extern "C" int omega4_bass_bars(int device, void* stream, int mem, const float* 
                                 float* bars_out) {
     if (!magnitudes || !bar_bins || !comp || !bars_out || n_ch < 0 || n_frames < 0 || n_bins <= 0 || n_bars <= 0 || n_bars > 128)
         return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_ch == 0 || n_frames == 0) return OMEGA4_OK;
     for (int b = 0; b < n_bars; ++b)
         if (bar_bins[2 * b] < 0 || bar_bins[2 * b + 1] < 0 || bar_bins[2 * b] + bar_bins[2 * b + 1] > n_bins)
             return fail(OMEGA4_ERR_INVALID, "bar bins out of range");
-    if (omega4_device_count() == 0) return fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback");
-    CK(cudaSetDevice(device));
-    cudaStream_t s = (cudaStream_t)stream;
-    std::vector<void*> to_free;
-    auto cleanup = [&]() { for (void* q : to_free) cudaFree(q); };
-#define CKF(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) { cleanup(); return fail(OMEGA4_ERR_CUDA, std::string(#expr " failed: ") + cudaGetErrorString(e__)); } } while (0)
-    int* d_bins = nullptr; float* d_comp = nullptr;
-    CKF(cudaMalloc(&d_bins, (size_t)n_bars * 2 * sizeof(int))); to_free.push_back(d_bins);
-    CKF(cudaMalloc(&d_comp, (size_t)n_bars * sizeof(float))); to_free.push_back(d_comp);
-    CKF(cudaMemcpyAsync(d_bins, bar_bins, (size_t)n_bars * 2 * sizeof(int), cudaMemcpyHostToDevice, s));
-    CKF(cudaMemcpyAsync(d_comp, comp, (size_t)n_bars * sizeof(float), cudaMemcpyHostToDevice, s));
-    const float* d_mag = magnitudes; float* d_out = bars_out; float* d_state = state;
-    const size_t rows = (size_t)n_ch * n_frames;
-    if (mem == OMEGA4_MEM_HOST) {
-        float* t = nullptr;
-        CKF(cudaMalloc(&t, rows * n_bins * sizeof(float))); to_free.push_back(t);
-        CKF(cudaMemcpyAsync(t, magnitudes, rows * n_bins * sizeof(float), cudaMemcpyHostToDevice, s));
-        d_mag = t;
-        CKF(cudaMalloc(&d_out, rows * n_bars * sizeof(float))); to_free.push_back(d_out);
-        if (state) {
-            CKF(cudaMalloc(&d_state, (size_t)n_ch * n_bars * sizeof(float))); to_free.push_back(d_state);
-            CKF(cudaMemcpyAsync(d_state, state, (size_t)n_ch * n_bars * sizeof(float), cudaMemcpyHostToDevice, s));
-        }
-    } else if (mem != OMEGA4_MEM_DEVICE) {
-        cleanup();
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
-    }
-    bass_bars_kernel<<<(unsigned)((n_ch + 3) / 4), 128, 0, s>>>(d_mag, n_ch, n_frames, n_bins, d_bins, d_comp, n_bars, d_state, d_out);
-    CKF(cudaGetLastError());
-    if (mem == OMEGA4_MEM_HOST) {
-        CKF(cudaMemcpyAsync(bars_out, d_out, rows * n_bars * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (state) CKF(cudaMemcpyAsync(state, d_state, (size_t)n_ch * n_bars * sizeof(float), cudaMemcpyDeviceToHost, s));
-    }
-    CKF(cudaStreamSynchronize(s));
-    cleanup();
-#undef CKF
-    return OMEGA4_OK;
+    if (int rc = use_device(device)) return rc;
+    const long long rows = (long long)n_ch * n_frames;
+    HostStage hs((cudaStream_t)stream, mem);
+    const int* d_bins; const float* d_comp; const float* d_mag; float* d_out; float* d_state;
+    int rc;
+    if ((rc = hs.table(bar_bins, 2LL * n_bars, &d_bins)) || (rc = hs.table(comp, n_bars, &d_comp)) ||
+        (rc = hs.in(magnitudes, rows * n_bins, &d_mag)) || (rc = hs.out(bars_out, rows * n_bars, &d_out)) ||
+        (rc = hs.inout(state, (long long)n_ch * n_bars, 0, &d_state)))
+        return rc;
+    bass_bars_kernel<<<(unsigned)((n_ch + 3) / 4), 128, 0, hs.s>>>(d_mag, n_ch, n_frames, n_bins, d_bins, d_comp, n_bars, d_state, d_out);
+    CK(cudaGetLastError());
+    return hs.finish();
 }
 
 extern "C" int omega4_synth_fill(int device, void* stream, float* out_device, int n_streams, int n_channels,
@@ -2064,8 +2042,7 @@ extern "C" int omega4_synth_fill(int device, void* stream, float* out_device, in
     if (!out_device || n_streams < 0 || n_channels <= 0 || n_samples < 0 || row_stride < n_samples || sample_rate <= 0)
         return fail(OMEGA4_ERR_INVALID, "bad arguments");
     if (n_streams == 0 || n_samples == 0) return OMEGA4_OK;
-    if (omega4_device_count() == 0) return fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback");
-    CK(cudaSetDevice(device));
+    if (int rc = use_device(device)) return rc;
     const int rows = n_streams * n_channels;
     if (rows > 65535) return fail(OMEGA4_ERR_INVALID, "too many rows for one synth launch (max 65535)");
     const double clip_s = (double)(clip_samples > 0 ? clip_samples : n_samples) / sample_rate;
@@ -2083,8 +2060,7 @@ extern "C" omega4_bars* omega4_bars_create(const omega4_bars_desc* d, int device
     if (!d || !d->bands || d->spectrum_len < 2 || d->n_bars < 1 || d->percentile < 0 || d->percentile > 100) {
         fail(OMEGA4_ERR_INVALID, "bad bars descriptor"); return nullptr;
     }
-    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return nullptr; }
-    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return nullptr; }
+    if (use_device(device)) return nullptr;
     omega4_bars* b = new omega4_bars();
     b->device = device; b->T = d->spectrum_len; b->scale = d->scale; b->normalize_max = d->normalize_max;
     int nv = 0;
@@ -2115,7 +2091,7 @@ extern "C" void omega4_bars_destroy(omega4_bars* b) {
     if (!b) return;
     cudaSetDevice(b->device);
     cudaFree(b->bands); cudaFree(b->gain); cudaFree(b->sf); cudaFree(b->sfc);
-    b->h_spec.release(); b->h_out.release(); b->h_peak.release(); b->h_state.release(); b->state_in.release();
+    b->stage.release(); b->state_in.release();
     cudaGetLastError();
     delete b;
 }
@@ -2125,56 +2101,26 @@ extern "C" int omega4_bars_count(const omega4_bars* b) { return b ? b->n_valid :
 extern "C" int omega4_bars_run(omega4_bars* b, void* stream, int mem, const float* spectrum, int n_ch, int n_hops,
                                float* state, int fresh, float* band_values, float* peak_values) {
     if (!b || !spectrum || !band_values || n_ch < 0 || n_hops < 0) return fail(OMEGA4_ERR_INVALID, "bad arguments");
+    if (int rc = check_mem(mem)) return rc;
     if (n_ch == 0 || n_hops == 0) return OMEGA4_OK;
     CK(cudaSetDevice(b->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    const size_t rows = (size_t)n_ch * n_hops;
-    const size_t st_bytes = (size_t)n_ch * (1 + b->n_valid) * sizeof(float);
-    const float* d_spec = spectrum; float* d_out = band_values; float* d_peak = peak_values; float* d_state = state;
+    HostStage& hs = b->stage;
+    hs.begin((cudaStream_t)stream, mem);
+    const long long rows = (long long)n_ch * n_hops;
     const int is_fresh = (fresh || !state) ? 1 : 0;
-    if (mem == OMEGA4_MEM_HOST) {
-        int rc = b->h_spec.ensure(rows * b->T * sizeof(float)); if (rc) return rc;
-        rc = b->h_out.ensure(rows * b->n_valid * sizeof(float)); if (rc) return rc;
-        CK(cudaMemcpyAsync(b->h_spec.p, spectrum, rows * b->T * sizeof(float), cudaMemcpyHostToDevice, s));
-        d_spec = (const float*)b->h_spec.p; d_out = (float*)b->h_out.p;
-        if (peak_values) { rc = b->h_peak.ensure(rows * b->n_valid * sizeof(float)); if (rc) return rc; d_peak = (float*)b->h_peak.p; }
-        if (state) {
-            rc = b->h_state.ensure(st_bytes); if (rc) return rc;
-            if (!is_fresh) CK(cudaMemcpyAsync(b->h_state.p, state, st_bytes, cudaMemcpyHostToDevice, s));
-            d_state = (float*)b->h_state.p;
-        }
-    } else if (mem != OMEGA4_MEM_DEVICE) {
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
-    }
-    {
-        int rc = bars_launch(b, s, d_spec, n_ch, n_hops, d_state, is_fresh, d_out, d_peak, &b->state_in);
-        if (rc) return rc;
-    }
-    if (mem == OMEGA4_MEM_HOST) {
-        CK(cudaMemcpyAsync(band_values, d_out, rows * b->n_valid * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (peak_values) CK(cudaMemcpyAsync(peak_values, d_peak, rows * b->n_valid * sizeof(float), cudaMemcpyDeviceToHost, s));
-        if (state) CK(cudaMemcpyAsync(state, d_state, st_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-    }
-    return OMEGA4_OK;
+    const float* d_spec; float* d_out; float* d_peak; float* d_state;
+    int rc;
+    if ((rc = hs.in(spectrum, rows * b->T, &d_spec)) || (rc = hs.out(band_values, rows * b->n_valid, &d_out)) ||
+        (rc = hs.out(peak_values, rows * b->n_valid, &d_peak)) ||
+        (rc = hs.inout(state, (long long)n_ch * (1 + b->n_valid), is_fresh, &d_state)) ||
+        (rc = bars_launch(b, hs.s, d_spec, n_ch, n_hops, d_state, is_fresh, d_out, d_peak, &b->state_in)))
+        return rc;
+    return hs.finish();
 }
 
 // ------------------------------------------------------------------------------------------
 // block meters (loudness, one-third-octave, sound level meter): the host side their calls share
 // ------------------------------------------------------------------------------------------
-// create: a meter object needs a device, made current here
-static bool meter_device(int device) {
-    if (omega4_device_count() == 0) { fail(OMEGA4_ERR_NO_DEVICE, "no CUDA device visible: libomega4_cuda has no CPU fallback"); return false; }
-    if (cudaSetDevice(device) != cudaSuccess) { fail(OMEGA4_ERR_CUDA, "cudaSetDevice failed"); return false; }
-    return true;
-}
-
-static int check_mem(int mem) {
-    if (mem != OMEGA4_MEM_HOST && mem != OMEGA4_MEM_DEVICE)
-        return fail(OMEGA4_ERR_INVALID, "mem must be OMEGA4_MEM_HOST or OMEGA4_MEM_DEVICE");
-    return OMEGA4_OK;
-}
-
 // the push arguments every block meter takes (include/omega4_cuda.h); `outs` are its float outputs, null or not
 static int check_push(const void* h, int mem, const float* samples, long long ch_stride, int n_rows,
                       long long n_samples, const double* state, long long out_stride,
@@ -2188,81 +2134,12 @@ static int check_push(const void* h, int mem, const float* samples, long long ch
     return OMEGA4_OK;
 }
 
-// OMEGA4_MEM_HOST staging of one call: its host inputs go to device buffers the meter keeps (they only grow), the
-// kernels run on those, and finish() copies the outputs and the state back and synchronises once.  Sizes and
-// pitches are in floats.
-struct HostStage {
-    struct Back { float* dst; long long dpitch; const float* src; long long width, rows; };
-    DevBuf buf[5];                 // slot k holds the k-th array a call stages; a push with three outputs uses all
-    Back back[3];
-    int nbuf = 0, nback = 0;
-    cudaStream_t s = nullptr;
-    double* state = nullptr;       // host state to copy back, from state_dev
-    const double* state_dev = nullptr;
-    size_t state_bytes = 0;
-
-    void begin(cudaStream_t stream) { s = stream; nbuf = nback = 0; state = nullptr; }
-
-    // the block count of a push of n samples: floor((T + n) / sub) - floor(T / sub), with T = state[0] common to
-    // the rows of one state array and readable on the host
-    static long long blocks(const double* st, int fresh, long long n, int sub) {
-        const long long T = fresh ? 0 : (long long)st[0];
-        return (T + n) / sub - T / sub;
-    }
-
-    // rows x width floats at src (row pitch spitch) -> a dense device copy
-    int in(const float* src, long long spitch, long long width, long long rows, const float** dev) {
-        DevBuf& b = buf[nbuf++];
-        const size_t bytes = (size_t)(width * rows) * sizeof(float);
-        if (int rc = b.ensure(bytes ? bytes : sizeof(float))) return rc;
-        if (bytes) CK(cudaMemcpy2DAsync(b.p, width * sizeof(float), src, spitch * sizeof(float), width * sizeof(float),
-                                        rows, cudaMemcpyHostToDevice, s));
-        *dev = (const float*)b.p;
-        return OMEGA4_OK;
-    }
-
-    // a device buffer of rows x width floats that finish() copies to dst (row pitch dpitch); nullptr when dst is
-    // null or there is nothing to write
-    int out(float* dst, long long dpitch, long long width, long long rows, float** dev) {
-        DevBuf& b = buf[nbuf++];
-        *dev = nullptr;
-        if (!dst || width * rows == 0) return OMEGA4_OK;
-        if (int rc = b.ensure((size_t)(width * rows) * sizeof(float))) return rc;
-        *dev = (float*)b.p;
-        back[nback++] = {dst, dpitch, *dev, width, rows};
-        return OMEGA4_OK;
-    }
-
-    // a push's inputs: the samples [rows][n] (row pitch *ch_stride) densely, and the carried state (copied in
-    // unless fresh, back at finish()); the pointers and the stride are replaced by the device ones
-    int push(const float** x, long long* ch_stride, long long rows, long long n, double** st, size_t st_bytes,
-             int fresh) {
-        if (int rc = in(*x, *ch_stride, n, rows, x)) return rc;
-        *ch_stride = n;
-        DevBuf& b = buf[nbuf++];
-        if (int rc = b.ensure(st_bytes)) return rc;
-        if (!fresh) CK(cudaMemcpyAsync(b.p, *st, st_bytes, cudaMemcpyHostToDevice, s));
-        state = *st; state_dev = (const double*)b.p; state_bytes = st_bytes;
-        *st = (double*)b.p;
-        return OMEGA4_OK;
-    }
-
-    int finish() {
-        for (int i = 0; i < nback; ++i) {
-            const Back& c = back[i];
-            if (c.dpitch == c.width)
-                CK(cudaMemcpyAsync(c.dst, c.src, (size_t)(c.width * c.rows) * sizeof(float), cudaMemcpyDeviceToHost, s));
-            else
-                CK(cudaMemcpy2DAsync(c.dst, c.dpitch * sizeof(float), c.src, c.width * sizeof(float),
-                                     c.width * sizeof(float), c.rows, cudaMemcpyDeviceToHost, s));
-        }
-        if (state) CK(cudaMemcpyAsync(state, state_dev, state_bytes, cudaMemcpyDeviceToHost, s));
-        CK(cudaStreamSynchronize(s));
-        return OMEGA4_OK;
-    }
-
-    void release() { for (DevBuf& b : buf) b.release(); }
-};
+// the block count of a push of n samples: floor((T + n) / sub) - floor(T / sub), with T = state[0] common to the rows
+// of one state array and readable on the host in OMEGA4_MEM_HOST mode
+static long long push_blocks(const double* st, int fresh, long long n, int sub) {
+    const long long T = fresh ? 0 : (long long)st[0];
+    return (T + n) / sub - T / sub;
+}
 
 // ------------------------------------------------------------------------------------------
 // ITU-R BS.1770-4 program loudness / EBU Tech 3342 loudness range (extension outside reference parity)
@@ -2300,7 +2177,7 @@ extern "C" omega4_loudness* omega4_loudness_create(const omega4_loudness_desc* d
         if (!(fabs(a[2]) < 1.0) || !(fabs(a[1]) < 1.0 + a[2])) {
             fail(OMEGA4_ERR_INVALID, "K-weighting biquads must have their poles inside the unit circle"); return nullptr;
         }
-    if (!meter_device(device)) return nullptr;
+    if (use_device(device)) return nullptr;
     omega4_loudness* h = new omega4_loudness();
     h->device = device; h->fs = d->sample_rate; h->C = d->channels; h->sub = d->sub;
     const double q[10] = {d->shelf_b[0], d->shelf_b[1], d->shelf_b[2], d->shelf_a[1], d->shelf_a[2],
@@ -2353,17 +2230,18 @@ extern "C" int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, c
     if ((rc = h->Z.ensure((size_t)n_streams * nsegb * sizeof(double)))) return rc;
     a.E = (double*)h->E.p; a.P = (float*)h->P.p; a.FS = (double*)h->FS.p; a.Z = (double*)h->Z.p;
     HostStage& hs = h->stage;
+    hs.begin(s, mem);
     if (mem == OMEGA4_MEM_HOST) {
-        const long long ndone = HostStage::blocks(state, fresh, n_samples, h->sub);
+        const long long ndone = push_blocks(state, fresh, n_samples, h->sub);
         if ((momentary || short_term) && out_stride < ndone)
             return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
-        hs.begin(s);
-        if ((rc = hs.push(&a.x, &a.ch_stride, rows, n_samples, &a.state, (size_t)n_streams * SD * sizeof(double), fresh)) ||
+        if ((rc = hs.in(samples, ch_stride, n_samples, rows, &a.x)) ||
+            (rc = hs.inout(state, (long long)n_streams * SD, fresh, &a.state)) ||
             (rc = hs.out(momentary, out_stride, ndone, n_streams, &a.mom)) ||
             (rc = hs.out(short_term, out_stride, ndone, n_streams, &a.st)) ||
             (rc = hs.out(sample_peak, rows, rows, 1, &a.peak_db)))
             return rc;
-        a.out_stride = ndone;
+        a.ch_stride = n_samples; a.out_stride = ndone;
     }
     const long long warps = (rows * ((nsegb + LOUD_GROUP - 1) / LOUD_GROUP) + 31) / 32;
     loudness_chain_kernel<<<(unsigned)((warps + LOUD_WARPS - 1) / LOUD_WARPS), LOUD_WARPS * 32, 0, s>>>(a);
@@ -2371,7 +2249,7 @@ extern "C" int omega4_loudness_push(omega4_loudness* h, void* stream, int mem, c
     loudness_finalize_kernel<<<(unsigned)((n_streams + LOUD_WARPS - 1) / LOUD_WARPS), LOUD_WARPS * 32, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 2;
-    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
+    return hs.finish();
 }
 
 extern "C" int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem, const float* momentary,
@@ -2381,22 +2259,18 @@ extern "C" int omega4_loudness_summary(omega4_loudness* h, void* stream, int mem
     if (int rc = check_mem(mem)) return rc;
     if (n_streams == 0) return OMEGA4_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    const float* m = momentary; const float* st = short_term; float* o = out;
-    long long ld = stride;
     HostStage& hs = h->stage;
-    if (mem == OMEGA4_MEM_HOST) {
-        hs.begin(s);
-        int rc;
-        if ((rc = hs.in(momentary, stride, n_steps, n_streams, &m)) ||
-            (rc = hs.in(short_term, stride, n_steps, n_streams, &st)) || (rc = hs.out(out, 4, 4, n_streams, &o)))
-            return rc;
-        ld = n_steps;
-    }
-    loudness_summary_kernel<<<(unsigned)n_streams, LOUD_SUM_THREADS, 0, s>>>(m, st, ld, n_steps, o);
+    hs.begin((cudaStream_t)stream, mem);
+    const float* m; const float* st; float* o;
+    int rc;
+    if ((rc = hs.in(momentary, stride, n_steps, n_streams, &m)) ||
+        (rc = hs.in(short_term, stride, n_steps, n_streams, &st)) || (rc = hs.out(out, 4, 4, n_streams, &o)))
+        return rc;
+    const long long ld = hs.host ? n_steps : stride;
+    loudness_summary_kernel<<<(unsigned)n_streams, LOUD_SUM_THREADS, 0, hs.s>>>(m, st, ld, n_steps, o);
     CK(cudaGetLastError());
     h->launches += 1;
-    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
+    return hs.finish();
 }
 
 // ------------------------------------------------------------------------------------------
@@ -2454,7 +2328,7 @@ extern "C" omega4_octave* omega4_octave_create(const omega4_octave_desc* d, int 
     }
     table[d->n_bands * OCT_COEF + 6] = 2.0 / d->sub;      // the overall column: no filter, unit gain
     table[d->n_bands * OCT_COEF + 7] = 2.0;
-    if (!meter_device(device)) return nullptr;
+    if (use_device(device)) return nullptr;
     omega4_octave* h = new omega4_octave();
     h->device = device; h->fs = d->sample_rate; h->nb = d->n_bands; h->sub = d->sub;
     const int rc = h->coef.ensure(sizeof table);          // sets the error message itself when it fails
@@ -2495,22 +2369,23 @@ extern "C" int omega4_octave_push(omega4_octave* h, void* stream, int mem, const
     a.state = state; a.fresh = fresh ? 1 : 0;
     a.levels = levels; a.out_stride = out_stride; a.leq = leq; a.lmax = lmax;
     HostStage& hs = h->stage;
+    hs.begin(s, mem);
     if (mem == OMEGA4_MEM_HOST) {
-        const long long ndone = HostStage::blocks(state, fresh, n_samples, h->sub);
+        const long long ndone = push_blocks(state, fresh, n_samples, h->sub);
         if (levels && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
-        hs.begin(s);
         const long long cols = (long long)n_rows * ncol;
         int rc;
-        if ((rc = hs.push(&a.x, &a.ch_stride, n_rows, n_samples, &a.state, (size_t)n_rows * SD * sizeof(double), fresh)) ||
+        if ((rc = hs.in(samples, ch_stride, n_samples, n_rows, &a.x)) ||
+            (rc = hs.inout(state, (long long)n_rows * SD, fresh, &a.state)) ||
             (rc = hs.out(levels, out_stride * ncol, ndone * ncol, n_rows, &a.levels)) ||
             (rc = hs.out(leq, cols, cols, 1, &a.leq)) || (rc = hs.out(lmax, cols, cols, 1, &a.lmax)))
             return rc;
-        a.out_stride = ndone;
+        a.ch_stride = n_samples; a.out_stride = ndone;
     }
     octave_kernel<<<(unsigned)((n_rows + OCT_WARPS - 1) / OCT_WARPS), OCT_WARPS * 32, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 1;
-    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
+    return hs.finish();
 }
 
 // ------------------------------------------------------------------------------------------
@@ -2564,7 +2439,7 @@ extern "C" omega4_slm* omega4_slm_create(const omega4_slm_desc* d, int device) {
     }
     w[2].g2 = 1.0;                                          // Z: no filter
     for (SlmCoef& c : w) c.g2_sub = c.g2 / d->sub;
-    if (!meter_device(device)) return nullptr;
+    if (use_device(device)) return nullptr;
     omega4_slm* h = new omega4_slm();
     h->device = device; h->fs = d->sample_rate; h->sub = d->sub;
     h->aF = exp(-1.0 / (0.125 * d->sample_rate));
@@ -2601,23 +2476,23 @@ extern "C" int omega4_slm_push(omega4_slm* h, void* stream, int mem, const float
     a.state = state; a.fresh = fresh ? 1 : 0;
     a.levels = levels; a.out_stride = out_stride; a.totals = totals;
     HostStage& hs = h->stage;
+    hs.begin(s, mem);
     if (mem == OMEGA4_MEM_HOST) {
-        const long long ndone = HostStage::blocks(state, fresh, n_samples, h->sub);
+        const long long ndone = push_blocks(state, fresh, n_samples, h->sub);
         if (levels && out_stride < ndone) return fail(OMEGA4_ERR_INVALID, "out_stride below the block count of this push");
-        hs.begin(s);
         const long long tot = (long long)n_rows * SLM_NW * SLM_NTOT;
         int rc;
-        if ((rc = hs.push(&a.x, &a.ch_stride, n_rows, n_samples, &a.state,
-                          (size_t)n_rows * SLM_STATE_DOUBLES * sizeof(double), fresh)) ||
+        if ((rc = hs.in(samples, ch_stride, n_samples, n_rows, &a.x)) ||
+            (rc = hs.inout(state, (long long)n_rows * SLM_STATE_DOUBLES, fresh, &a.state)) ||
             (rc = hs.out(levels, out_stride * SLM_NCOL, ndone * SLM_NCOL, n_rows, &a.levels)) ||
             (rc = hs.out(totals, tot, tot, 1, &a.totals)))
             return rc;
-        a.out_stride = ndone;
+        a.ch_stride = n_samples; a.out_stride = ndone;
     }
     slm_kernel<<<(unsigned)((n_rows + SLM_ROWS - 1) / SLM_ROWS), SLM_NW * 32, 0, s>>>(a);
     CK(cudaGetLastError());
     h->launches += 1;
-    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
+    return hs.finish();
 }
 
 extern "C" int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, const float* levels, int n_rows,
@@ -2640,19 +2515,16 @@ extern "C" int omega4_slm_percentiles(omega4_slm* h, void* stream, int mem, cons
     }
     if (n_rows == 0) return OMEGA4_OK;
     CK(cudaSetDevice(h->device));
-    cudaStream_t s = (cudaStream_t)stream;
-    a.levels = levels; a.stride = stride; a.n_steps = n_steps; a.column = column; a.n_pct = n_pct; a.out = out;
+    a.n_steps = n_steps; a.column = column; a.n_pct = n_pct;
     HostStage& hs = h->stage;
-    if (mem == OMEGA4_MEM_HOST) {
-        hs.begin(s);
-        int rc;
-        if ((rc = hs.in(levels, stride * SLM_NCOL, (long long)n_steps * SLM_NCOL, n_rows, &a.levels)) ||
-            (rc = hs.out(out, n_pct, n_pct, n_rows, &a.out)))
-            return rc;
-        a.stride = n_steps;
-    }
-    slm_percentile_kernel<<<(unsigned)n_rows, SLM_PCT_THREADS, 0, s>>>(a);
+    hs.begin((cudaStream_t)stream, mem);
+    int rc;
+    if ((rc = hs.in(levels, stride * SLM_NCOL, (long long)n_steps * SLM_NCOL, n_rows, &a.levels)) ||
+        (rc = hs.out(out, n_pct, n_pct, n_rows, &a.out)))
+        return rc;
+    a.stride = hs.host ? n_steps : stride;
+    slm_percentile_kernel<<<(unsigned)n_rows, SLM_PCT_THREADS, 0, hs.s>>>(a);
     CK(cudaGetLastError());
     h->launches += 1;
-    return mem == OMEGA4_MEM_HOST ? hs.finish() : OMEGA4_OK;
+    return hs.finish();
 }

@@ -15,6 +15,8 @@
  *   - `mem` says where the DATA pointers of that call live (samples, frames, outputs).  Table
  *     pointers in omega4_plan_desc are always host memory and are copied at plan creation.
  *   - sample/frame pointers must be 16-byte aligned in device mode.
+ *   - one call at a time per plan, bars or meter object: it owns its scratch and OMEGA4_MEM_HOST staging buffers.
+ *     The plan-less entry points free what they stage before they return.
  */
 #ifndef OMEGA4_CUDA_H
 #define OMEGA4_CUDA_H
@@ -312,8 +314,7 @@ int omega4_bars_run(omega4_bars* bars, void* stream, int mem, const float* spect
  *              knows the count without a sync.  Blocks at column >= out_stride are not written (in host mode an
  *              out_stride below the count is an error).
  *   alignment  samples and every float output float-aligned (no wider alignment is needed), state double-aligned
- * Tile lengths are arbitrary (no multiple of sub or of 512 needed).  One call at a time per object: it owns its
- * scratch and OMEGA4_MEM_HOST staging buffers. */
+ * Tile lengths are arbitrary (no multiple of sub or of 512 needed). */
 
 /* ---- ITU-R BS.1770-4 program loudness and EBU Tech 3342 loudness range (extension) ---------- */
 /* Not part of the reference's behaviour: ProfessionalMetering (omega4_analyze's five meters) is not textbook
